@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port, all host cores)
+  python bench.py --steps K --dump-outputs DIR             # + what the last timed step computed, as DIR/*.npy
 
 Workload (BASELINE.json configs[1]): 1M users / 200k recipes / 95 labels, D=128, BPR
 triples (uniform users, Zipf(1.05) positives, uniform negatives), Adam with TF-1.x
@@ -237,7 +238,7 @@ def run_reference(args, cfg, B):
     lab = synth.make_user_label_csr(U, L)
     port = CpuPort(P, R, Cat, G, Hyper(learner="adam", lr=0.001), threads=cores)
     del P
-    steps, warm = max(1, min(args.steps, 5)), max(1, min(args.warmup, 1))
+    steps, warm = args.steps, max(1, min(args.warmup, 1))
     bs = make_batches(cfg, B, steps + warm, 777, item_cats, lab, dense=True)
     T = lambda x, dt=None: torch.as_tensor(x if dt is None else x.astype(dt))
     t0 = None
@@ -933,6 +934,27 @@ def run_sharded(args, cfg, B):
 
 
 # ----------------------------------------------------------------------------- GPU arm
+DUMP_ROWS = {"P": 8192, "R": 16384}      # sampled rows of the two large tables: 21 MB + 8 MB at D=128
+
+
+def dump_outputs(out_dir, eng):
+    """--dump-outputs: what the last timed step hands its caller, as float32 DIR/<name>.npy -- the step's scalar
+    vector (FR_OUT_*: loss, norm, clip scale, ...) and the tables it updated: Category_Embedding and General_Memory
+    whole, Personal_Memory and Recipe_Embedding as a fixed seeded sample of rows (the full tables are GBs).  The
+    sample depends only on the table sizes, so two builds run with the same arguments compare row for row."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"scalars": eng.read_scalars()}
+    eng.flush()                          # lazy Adam: every row brought to the current step, as Engine.tables() does
+    for k, n in DUMP_ROWS.items():
+        t = getattr(eng, k)
+        rows = np.sort(np.random.default_rng(2026).choice(t.shape[0], min(n, t.shape[0]), replace=False))
+        out[k + "_sample"] = t[torch.as_tensor(rows, device=t.device)].float().cpu().numpy()
+    out["Cat"], out["G"] = eng.Cat.float().cpu().numpy(), eng.G.float().cpu().numpy()
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float32))
+
+
 def run_ours(args, cfg, B):
     import torch
     import torch.distributed as dist
@@ -995,6 +1017,8 @@ def run_ours(args, cfg, B):
         t = torch.tensor([ms], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
     clk = clocks.stop()
     value = world * B * args.steps / (ms / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, eng)     # before the legs below train the same tables further
 
     # ---- per-kernel timing (CUDA events inside fr_train_step, on its stream), same steps again
     eng.timing_enable(True)
@@ -1247,7 +1271,14 @@ def main():
     ap.add_argument("--no-catalog", action="store_true", help="skip the full-catalog top-K legs")
     ap.add_argument("--learner", default="adam", help="adam (reference default) | adagrad | rmsprop | sgd")
     ap.add_argument("--adam-mode", default="lazy", choices=["lazy", "lazy_exact", "dense"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to "
+                    "DIR/<name>.npy (float32, ~30 MB: step scalars, Cat, G, a fixed sample of P and R rows), so that two "
+                    "builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs covers the single-process GPU run (--impl ours without torchrun)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = SMALL if args.small else (CFG3 if args.cfg3 else CFG2)
     if args.cfg3 and int(os.environ.get("WORLD_SIZE", "1")) < 8:

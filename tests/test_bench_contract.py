@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -20,17 +21,48 @@ def last_json_line(text):
 
 
 def test_reference_arm_runs_and_prints_the_contract_line():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--small", "--steps", "1",
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--small", "--steps", "6",
                         "--warmup", "1", "--batch", "4096"], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, r.stderr[-2000:]
     d = last_json_line(r.stdout)
-    assert BASE_KEYS <= set(d) and d["impl"] == "reference"
+    assert BASE_KEYS <= set(d) and d["impl"] == "reference" and d["steps"] == 6
     assert d["metric"] == "bpr_train_triples_per_sec" and d["unit"] == "triples/s" and d["higher_is_better"] is True
     assert d["vs_baseline"] is None and d["value"] > 0
     cb = d["cpu_baseline"]
     assert cb["kind"] in ("port", "reference") and cb["cores"] >= 1 and cb["sample"] and cb["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in d["config"] and "model" not in d["config"]
+
+
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]])
+def test_bench_refuses_what_it_cannot_do(extra):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                       timeout=120, cwd=ROOT)
+    assert r.returncode == 2 and "error:" in r.stderr, r.stderr[-2000:]
+
+
+@pytest.mark.gpu
+def test_dump_outputs_writes_the_last_timed_step(tmp_path):
+    """--dump-outputs: float32 arrays of what the last timed step computed, 64 MB at most.  The same arguments give the
+    same inputs, so a second run writes the same arrays (to summation order)."""
+    from tests.util import assert_close
+    runs = [tmp_path / "a", tmp_path / "b"]
+    for out in runs:
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--small", "--steps", "3", "--warmup", "3",
+                            "--preroll", "2", "--no-cpu", "--no-catalog", "--no-cfg5", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert last_json_line(r.stdout)["steps"] == 3
+    names = sorted(p.name for p in runs[0].iterdir())
+    assert names == ["Cat.npy", "G.npy", "P_sample.npy", "R_sample.npy", "scalars.npy"]
+    assert sum(p.stat().st_size for p in runs[0].iterdir()) <= 64 << 20
+    for n in names:
+        a, b = np.load(runs[0] / n), np.load(runs[1] / n)
+        assert a.dtype == np.float32 and np.isfinite(a).all(), n
+        if n == "scalars.npy":
+            np.testing.assert_allclose(b, a, rtol=1e-5, atol=0, err_msg=n)
+        else:
+            assert_close(b, a, what=n)
 
 
 @pytest.mark.parametrize("path", sorted(glob.glob(os.path.join(ROOT, "profiles", "r02_bench_*gpu.json"))))
