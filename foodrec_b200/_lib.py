@@ -85,6 +85,8 @@ _PROTOS = {
     "fr_catalog_prepare": (C.c_int, [C.c_void_p, C.POINTER(fr_catalog_opts), C.c_void_p, C.c_void_p]),
     "fr_catalog_topk": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                   C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_catalog_topk_excluding": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                            C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fr_gather_user_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "fr_catalog_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                    C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -37,7 +37,7 @@ struct CatalogWs {
   // per-pass workspace
   int mp_cap = 0;
   __nv_bfloat16* A = nullptr; float *bias = nullptr, *margin2 = nullptr, *cand_sc = nullptr;
-  int32_t *cand_row = nullptr, *cand_cnt = nullptr, *ovf = nullptr, *ovf_list = nullptr, *ovf_count = nullptr;
+  int32_t *cand_row = nullptr, *cand_cnt = nullptr, *ovf = nullptr, *ovf_list = nullptr, *ovf_count = nullptr, *keff = nullptr;
   double* scratch = nullptr; int exact_blocks = 0;
   unsigned long long* dbg = nullptr;
   uint32_t* ukeys = nullptr; SortBufs sortU; int32_t* block_first = nullptr;   // users sorted by best mask group
@@ -131,6 +131,21 @@ __device__ __forceinline__ const float4* user_row(const UserSrc& s, int j, int D
   return s.P + (size_t)user_of(s, j) * 5 * DV;
 }
 
+// Exclusion lists (catalog.cuh): CSR over query rows, ids in the OUTPUT id space (local row * id_mul + id_add).
+// An id is compared, never dereferenced: one this table cannot return (another shard's, out of range, negative) -> -1.
+struct ExclLists {
+  const int32_t* off;     // [n_users+1] or nullptr (no lists)
+  const int32_t* ids;     // [nnz]
+  int id_mul, id_add, n_items;
+};
+__device__ __forceinline__ int excl_local(const ExclLists& x, int id) {
+  const long long d = (long long)id - x.id_add;
+  if (d < 0) return -1;
+  const uint32_t u = (uint32_t)d, m = (uint32_t)x.id_mul;   // d < 2^32 (two int32s); 32-bit division stays inline
+  const uint32_t q = u / m;
+  return (u - q * m == 0 && q < (uint32_t)x.n_items) ? (int)q : -1;
+}
+
 // key of a query row = the mask group with the largest category term a/|g| * sum_{c in g} <P[u,0],Cat[c]>
 template <int NV>
 __global__ void __launch_bounds__(FR_THREADS)
@@ -172,7 +187,8 @@ __global__ void __launch_bounds__(FR_THREADS)
 cat_pack_users_kernel(UserSrc src, int n_rows, int m_pad, const float4* __restrict__ Cat, int DV, int KP, int a_split, float a,
                       float oma, int present, const float* __restrict__ rmax_p, float cfac,
                       __nv_bfloat16* __restrict__ A, float* __restrict__ bias, float* __restrict__ margin2,
-                      int32_t* __restrict__ block_first, int block_rows
+                      int32_t* __restrict__ block_first, int block_rows, ExclLists excl, int K,
+                      int32_t* __restrict__ keff, int32_t* __restrict__ ovf
 #ifdef FR_CAT_TILE_BOUND
                       , float* __restrict__ margin2r
 #endif
@@ -181,6 +197,17 @@ cat_pack_users_kernel(UserSrc src, int n_rows, int m_pad, const float4* __restri
   const int j = blockIdx.x * FR_WARPS_PER_BLOCK + (threadIdx.x >> 5);
   if (j >= m_pad) return;
   const bool valid = j < n_rows;
+  // K_eff of the row (in pass order, after the user sort): K + the listed ids that map into this table.  A row
+  // whose K_eff exceeds CAT_MAXK is flagged to the exact fallback here (this also clears ovf for the pass).
+  int ke = K;
+  if (valid && excl.off) {
+    const int qr = query_row(src, j);
+    const int e0 = __ldg(excl.off + qr), e1 = __ldg(excl.off + qr + 1);
+    int c = 0;
+    for (int e = e0 + lane; e < e1; e += 32) c += excl_local(excl, __ldg(excl.ids + e)) >= 0 ? 1 : 0;
+    ke += __reduce_add_sync(FR_FULL, c);
+  }
+  if (lane == 0) { keff[j] = min(ke, CAT_MAXK); ovf[j] = ke > CAT_MAXK ? 1 : 0; }
   float4 pr[5][NV];
   double h[4] = {0, 0, 0, 0};
   if (valid) {
@@ -342,6 +369,8 @@ struct FinParams {
   const float* margin2r; const float* tile_rho; int bn_shift;
 #endif
   const int32_t* ovf; int32_t* ovf_list; int32_t* ovf_count;
+  const int32_t* keff;                      // [m_pad] per-row K_eff
+  ExclLists excl;                           // carries id_mul / id_add of the outputs too
   int id_mul, id_add;
   int32_t* out_ids; double* out_scores;     // [n_users, K]
 };
@@ -364,6 +393,7 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
 
   bool overflow = f.ovf[row] != 0;
   int n_tot = 0;
+  const int Ke = f.keff[row];
   if (!overflow) {
     for (int sp = 0; sp < f.n_split; ++sp) {
       const size_t lr = (size_t)sp * f.m_pad + row;
@@ -376,12 +406,12 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
     }
     if (tid == 0) s_nF = 0;
     __syncthreads();
-    // tau = K-th largest approximate score over the union of the split lists
+    // tau = K_eff-th largest approximate score over the union of the split lists
     float lo = -__int_as_float(0x7f800000);
-    if (n_tot > f.K) {
+    if (n_tot > Ke) {
       // exact K-th largest key by 8-bit radix select over a shared-memory histogram: 4 passes x 3 barriers (the
       // bit-by-bit search it replaces cost 64 barriers and 32 sweeps over the list: 18 % of this kernel's instructions)
-      uint32_t res = 0; uint32_t need = (uint32_t)f.K;
+      uint32_t res = 0; uint32_t need = (uint32_t)Ke;
       for (int pass = 3; pass >= 0; --pass) {
         for (int b = tid; b < 256; b += FIN_THREADS) s_hist[b] = 0u;
         __syncthreads();
@@ -415,7 +445,7 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
         need = s_sel[1];
       }
 #ifdef FR_CAT_TILE_BOUND
-      lo = funkey(res);                 // K-th largest LOWER bound over the union of the lists
+      lo = funkey(res);                 // K_eff-th largest LOWER bound over the union of the lists
 #else
       lo = __fsub_rd(funkey(res), f.margin2[row]);
 #endif
@@ -433,6 +463,20 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
     __syncthreads();
     if (s_nF > CAT_FCAP) overflow = true;
   }
+  // The row's listed recipes of this table (local ids; at most K_eff - K <= CAT_MAXK - 1 of them here) are staged in
+  // the candidate area, free once the survivors are picked: s_ex[0] = count, s_ex[1..].  (No static shared memory is
+  // added: one more KB would cost this kernel a resident block per SM.)
+  int* s_ex = reinterpret_cast<int*>(csc);
+  if (!overflow && f.excl.off) {
+    if (tid == 0) s_ex[0] = 0;
+    __syncthreads();
+    const int qr = query_row(f.src, row);
+    const int e1 = __ldg(f.excl.off + qr + 1);
+    for (int e = __ldg(f.excl.off + qr) + tid; e < e1; e += FIN_THREADS) {
+      const int l = excl_local(f.excl, __ldg(f.excl.ids + e));
+      if (l >= 0) { const int pos = atomicAdd(s_ex, 1); if (pos < CAT_MAXK) s_ex[1 + pos] = l; }
+    }
+  }
   if (overflow) {                       // exact fallback takes this row
     if (tid == 0) { const int slot = atomicAdd(f.ovf_count, 1); f.ovf_list[slot] = row; }
     return;
@@ -447,10 +491,13 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
   __shared__ int s_masks;
   if (tid == 0) s_masks = 0;
   __syncthreads();
+  const int nex = f.excl.off ? min(s_ex[0], CAT_MAXK) : 0;
   for (int i = tid; i < nF; i += FIN_THREADS) {
     const int item = __ldg(f.row_item + frow[i]);
     const float4 m = __ldg(f.item_cats + item);
-    const int g = (m.x != 0.f ? 1 : 0) | (m.y != 0.f ? 2 : 0) | (m.z != 0.f ? 4 : 0) | (m.w != 0.f ? 8 : 0);
+    int g = (m.x != 0.f ? 1 : 0) | (m.y != 0.f ? 2 : 0) | (m.z != 0.f ? 4 : 0) | (m.w != 0.f ? 8 : 0);
+    for (int x = 0; x < nex; ++x)               // a listed survivor is scored like a recipe without a category: -inf
+      if (s_ex[1 + x] == item) { g = 0; break; }
     eid[i] = item;
     frow[i] = g;                                   // the padded row is no longer needed: keep the mask
     atomicOr(&s_masks, 1 << g);
@@ -571,6 +618,15 @@ __global__ void __launch_bounds__(EX_THREADS) cat_exact_kernel(const FinParams f
       }
     }
     __syncthreads();
+    if (f.excl.off) {                           // listed recipes leave the ranking (-inf is padded with -1 below)
+      const int qr = query_row(f.src, row);
+      const int e1 = __ldg(f.excl.off + qr + 1);
+      for (int e = __ldg(f.excl.off + qr) + tid; e < e1; e += EX_THREADS) {
+        const int l = excl_local(f.excl, __ldg(f.excl.ids + e));
+        if (l >= 0) sc[l] = -CUDART_INF;
+      }
+      __syncthreads();
+    }
     // radix select of the Keff-th largest 64-bit key
     unsigned long long prefix = 0;
     int need = Keff;
@@ -814,6 +870,7 @@ static int catalog_ensure_pass_ws(fr_ctx* h, CatalogWs& w, int mp) {
   if ((rc = dalloc(h, &w.cand_row, RL * CAT_CAP))) return rc;
   if ((rc = dalloc(h, &w.cand_cnt, RL))) return rc;
   if ((rc = dalloc(h, &w.ovf, R))) return rc;
+  if ((rc = dalloc(h, &w.keff, R))) return rc;
   if ((rc = dalloc(h, &w.ovf_list, R))) return rc;
   if ((rc = dalloc(h, &w.ovf_count, 1))) return rc;
   if ((rc = dalloc(h, &w.dbg, 8))) return rc;
@@ -828,11 +885,15 @@ static int catalog_ensure_pass_ws(fr_ctx* h, CatalogWs& w, int mp) {
   return FR_OK;
 }
 
-extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P_rows, int32_t n_users, int32_t K,
-                               int32_t id_mul, int32_t id_add, int32_t* out_ids, double* out_scores, fr_stream s) {
+extern "C" int fr_catalog_topk_excluding(fr_handle h, const int32_t* users, const float* P_rows, int32_t n_users, int32_t K,
+                                         const int32_t* excl_off, const int32_t* excl_ids, int32_t id_mul, int32_t id_add,
+                                         int32_t* out_ids, double* out_scores, fr_stream s) {
   if (!h || !out_ids || n_users < 0) return FR_ERR_ARG;
   if (!h->cat || !h->cat->prepared) return fail(h, FR_ERR_STATE, "fr_catalog_prepare first");
   if (K <= 0 || K > CAT_MAXK) return fail(h, FR_ERR_UNSUPPORTED, "K must be in [1,%d], got %d", CAT_MAXK, K);
+  if ((excl_off == nullptr) != (excl_ids == nullptr))
+    return fail(h, FR_ERR_ARG, "excl_off and excl_ids are given together (both NULL: no lists)");
+  if (excl_off && id_mul < 1) return fail(h, FR_ERR_ARG, "id_mul must be >= 1 with exclusion lists, got %d", id_mul);
   if (n_users == 0) return FR_OK;
   if (P_rows && h->health_blend) return fail(h, FR_ERR_ARG, "the health term needs user ids (labels): pass users, not dense P_rows");
   if (h->table_bf16) return fail(h, FR_ERR_UNSUPPORTED, "fr_catalog_* reads fp32 tables (exact fp64 re-rank): not available with bf16 tables");
@@ -864,6 +925,7 @@ extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P
     const int tps = std::max(1, (w.n_tiles + n_split - 1) / n_split);
     UserSrc src{reinterpret_cast<const float4*>(P_rows ? P_rows : h->tab.P), P_rows ? nullptr : users, row0, nullptr, health_of(h),
                 (uint32_t)h->cfg.num_users};
+    const ExclLists excl{excl_off, excl_ids, id_mul, id_add, w.I};
 
     std::array<cudaEvent_t, 5>* ev = nullptr;
     if (timing) {
@@ -889,14 +951,15 @@ extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P
     const int pgrid = (m_pad + FR_WARPS_PER_BLOCK - 1) / FR_WARPS_PER_BLOCK;
     if (h->NV == 1)
       cat_pack_users_kernel<1><<<pgrid, FR_THREADS, 0, st>>>(src, rows, m_pad, Cat4, DV, w.KP, w.a_split, h->mc.a, h->mc.oma, w.present,
-                                                            w.rmax, cfac, w.A, w.bias, w.margin2, bf, BMC FR_CAT_M2R(w));
+                                                            w.rmax, cfac, w.A, w.bias, w.margin2, bf, BMC, excl, K, w.keff, w.ovf
+                                                            FR_CAT_M2R(w));
     else
       cat_pack_users_kernel<2><<<pgrid, FR_THREADS, 0, st>>>(src, rows, m_pad, Cat4, DV, w.KP, w.a_split, h->mc.a, h->mc.oma, w.present,
-                                                            w.rmax, cfac, w.A, w.bias, w.margin2, bf, BMC FR_CAT_M2R(w));
+                                                            w.rmax, cfac, w.A, w.bias, w.margin2, bf, BMC, excl, K, w.keff, w.ovf
+                                                            FR_CAT_M2R(w));
     ++g_launches;
     FR_CHECK_LAUNCH(h);
     FR_CUDA(h, cudaMemsetAsync(w.cand_cnt, 0, (size_t)n_lists * m_pad * 4, st));
-    FR_CUDA(h, cudaMemsetAsync(w.ovf, 0, (size_t)m_pad * 4, st));
     FR_CUDA(h, cudaMemsetAsync(w.ovf_count, 0, 4, st));
     if (ev) FR_CUDA(h, cudaEventRecord((*ev)[1], st));
 
@@ -905,7 +968,7 @@ extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P
       if ((rc = make_tmap(h, &tmA, w.A, (uint64_t)16 * m_pad, w.a_split ? 2 * w.KP : w.KP, CAT_BM))) return rc;
       CatGemmParams p{};
       p.m_blocks = m_blocks; p.m_pad = m_pad; p.n_rows = rows; p.n_split = n_split; p.tiles_per_split = tps;
-      p.n_tiles = w.n_tiles; p.k_blocks = w.k_blocks; p.K = K; p.a_split = w.a_split;
+      p.n_tiles = w.n_tiles; p.k_blocks = w.k_blocks; p.keff = w.keff; p.a_split = w.a_split;
       // diagnostics / tuning switches (environment; never needed for results): FOODREC_CATALOG_DEBUG = ceiling
       // measurements (catalog.cuh), _DENSE_MIN / _BOOT_TILES = epilogue regime knobs, _CYCLES = in-kernel cycle counters
       { const char* dm = getenv("FOODREC_CATALOG_DEBUG"); p.debug_mode = dm ? atoi(dm) : 0; }
@@ -937,7 +1000,7 @@ extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P
 #ifdef FR_CAT_TILE_BOUND
     f.margin2r = w.margin2r; f.tile_rho = w.tile_rho; f.bn_shift = w.BN == 256 ? 8 : 7;
 #endif
-    f.ovf = w.ovf; f.ovf_list = w.ovf_list; f.ovf_count = w.ovf_count;
+    f.ovf = w.ovf; f.ovf_list = w.ovf_list; f.ovf_count = w.ovf_count; f.keff = w.keff; f.excl = excl;
     f.id_mul = id_mul; f.id_add = id_add; f.out_ids = out_ids; f.out_scores = out_scores;
     const size_t fsm = (size_t)CAT_FCAP * (8 + 4 + 4) + 32 + (size_t)5 * D * 4 + (size_t)n_lists * CAT_CAP * 8 +
                        (size_t)16 * D * 8 + 8;      // + the per-mask fp64 user rows of the re-rank
@@ -961,6 +1024,11 @@ extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P
     if (ev) FR_CUDA(h, cudaEventRecord((*ev)[4], st));
   }
   return FR_OK;
+}
+
+extern "C" int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P_rows, int32_t n_users, int32_t K,
+                               int32_t id_mul, int32_t id_add, int32_t* out_ids, double* out_scores, fr_stream s) {
+  return fr_catalog_topk_excluding(h, users, P_rows, n_users, K, nullptr, nullptr, id_mul, id_add, out_ids, out_scores, s);
 }
 
 extern "C" int fr_catalog_merge(fr_handle h, const int32_t* ids, const double* scores, int32_t n_lists,

@@ -19,6 +19,15 @@
 // bound is PER TILE: one heavy recipe (a hot item after training) widens the margin of its own 256-recipe tile only.
 // The survivors (K + a few dozen) are re-scored in fp64 from the fp32 tables and ranked by (score desc, id asc).  Rows
 // whose candidate list overflows (massive ties) fall back to an exact full scan.
+//
+// Exclusion lists (fr_catalog_topk_excluding): a query row may list recipe ids it must not get back (the user's
+// training positives).  The filter still runs over ALL recipes, with a per-row K_eff = K + (entries of the row's list
+// that map into this table; duplicates counted, which only widens the filter): tau_eff = the K_eff-th largest lower
+// bound.  At most K_eff - K of the K_eff largest lower bounds belong to listed recipes, so at least K UNLISTED recipes
+// have true score >= lower bound >= tau_eff: the K-th best unlisted score is >= tau_eff >= tau_run at any time, and a
+// member of the exact unlisted top-K has upper bound >= its score >= tau_run -- it is kept.  Listed survivors are then
+// dropped where scores are exact (the fp64 re-rank, or -inf in the exact fallback's score row).  K_eff > CAT_MAXK:
+// the row goes to the exact fallback up front.
 #pragma once
 // Per-tile filter bound (default).  -DFR_CAT_GLOBAL_BOUND builds the round-1 filter whose margin uses the largest
 // recipe norm of the WHOLE catalog (kept for A/B runs: foodrec_b200._build.build_variant("globalbound", [...])).
@@ -49,7 +58,8 @@ struct CatGemmParams {
   int m_blocks;          // user blocks of CAT_BM * CG rows in this pass
   int m_pad;             // m_blocks * CAT_BM * CG
   int n_rows;            // valid user rows in this pass
-  int n_split, tiles_per_split, n_tiles, k_blocks, K;
+  int n_split, tiles_per_split, n_tiles, k_blocks;
+  const int32_t* keff;         // [m_pad] K_eff of each row: K + its listed recipes in this table, <= CAT_MAXK
   int boot_tiles;        // tiles of the bootstrap pass that seeds the thresholds (0: none); chunks recorded must fit a list
   int dense_min;         // rows of a warp with a hit in a chunk from which the per-lane (shared staging) resolution is used
   int a_split;           // 1: A = bf16 head + bf16 tail (two MMAs per B block; needs 2*k_blocks <= CAT_KB_MAX)

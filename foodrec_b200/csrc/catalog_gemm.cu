@@ -47,8 +47,8 @@ __device__ __forceinline__ int sweep_tile(const int i, const int lo, const int h
   return r < lo ? r : r + len;
 }
 // A sweep is preceded by a BOOTSTRAP over its first `boot` tiles: the epilogue only records the maximum of every
-// 32-column chunk (no pushes).  K distinct chunk maxima are K distinct recipes, so the K-th largest of them is a
-// valid lower bound of the final K-th best score: the real sweep (which starts over at its first tile) begins with a
+// 32-column chunk (no pushes).  K_eff distinct chunk maxima are K_eff distinct recipes, so the K_eff-th largest of them
+// is a valid lower bound of the final K_eff-th best score (catalog.cuh: exclusion lists): the real sweep (which starts over at its first tile) begins with a
 // threshold near the top 1 % instead of -inf and skips the steep part of the ramp-up (~5x fewer pushes on a
 // 200k-recipe catalog for ~8 % more MMA work).  Extended index e in [0, boot + n): tile index = e < boot ? e : e - boot.
 struct SweepRange { int i0, i1, lo, hi, boot; };
@@ -77,14 +77,14 @@ __device__ __forceinline__ SweepRange sweep_range(const CatGemmParams& p, const 
   return r;
 }
 
-// Warp-collective compaction of lane L's candidate row: exact K-th largest of its entries by
+// Warp-collective compaction of lane L's candidate row: exact K_eff-th largest of its entries by
 // bitwise binary search (warp REDUX per bit), keep everything >= kth - 2E.  Returns lane L's new
 // (count, threshold); every other lane gets its own values back.
 struct CompactOut { int cnt; float thr; };
 __device__ __noinline__ CompactOut catalog_warp_compact(const int L, const int lane, float* __restrict__ cand_sc,
                                                         int32_t* __restrict__ cand_row, const size_t my_base,
                                                         const int my_cnt, const float my_thr, const float my_margin2,
-                                                        const int K, int32_t* ovf_flag, const bool drop_all
+                                                        const int my_K, int32_t* ovf_flag, const bool drop_all
 #ifdef FR_CAT_TILE_BOUND
                                                         , const float my_margin2r, const float* __restrict__ tile_rho,
                                                         const int bn_shift
@@ -94,6 +94,7 @@ __device__ __noinline__ CompactOut catalog_warp_compact(const int L, const int l
   const size_t base = __shfl_sync(FR_FULL, (unsigned long long)my_base, L);
   const int n = min(__shfl_sync(FR_FULL, my_cnt, L), CAT_CAP);
   const float m2 = __shfl_sync(FR_FULL, my_margin2, L);
+  const int K = __shfl_sync(FR_FULL, my_K, L);        // the row's K_eff (K + its listed recipes in this table)
   float sc[NV]; int32_t rw[NV]; uint32_t key[NV];
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
@@ -163,7 +164,7 @@ struct RowState {
 #define FR_CAT_ADJ(s) __fsub_rd((s).thr, (s).bias)
 #define FR_CAT_COMPACT_EXTRA(s, p)
 #endif
-  int cnt;
+  int cnt, K;              // K = the row's K_eff (catalog.cuh: exclusion lists widen the filter)
   size_t base;
   int32_t* ovf;
 };
@@ -267,7 +268,7 @@ __device__ __forceinline__ void catalog_filter_chunk(const float (&v)[32], const
   while (need) {
     const int L = __ffs(need) - 1;
     need &= need - 1;
-    const CompactOut o = catalog_warp_compact(L, lane, p.cand_sc, p.cand_row, s.base, s.cnt, s.thr, s.m2, p.K, s.ovf, false
+    const CompactOut o = catalog_warp_compact(L, lane, p.cand_sc, p.cand_row, s.base, s.cnt, s.thr, s.m2, s.K, s.ovf, false
                                               FR_CAT_COMPACT_EXTRA(s, p));
     s.cnt = o.cnt; s.thr = o.thr;
     s.adj = FR_CAT_ADJ(s);
@@ -422,7 +423,7 @@ catalog_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       const bool valid = grow < p.n_rows;
       const size_t list = (static_cast<size_t>(sp) * NSET + e) * p.m_pad + grow;
       RowState s;
-      s.base = list * CAT_CAP; s.m2 = __ldg(p.margin2 + grow); s.thr = (valid && p.debug_mode != 3) ? -INF : INF; s.cnt = 0; s.bias = 0.f;
+      s.base = list * CAT_CAP; s.m2 = __ldg(p.margin2 + grow); s.K = __ldg(p.keff + grow); s.thr = (valid && p.debug_mode != 3) ? -INF : INF; s.cnt = 0; s.bias = 0.f;
       s.adj = s.thr; s.ovf = p.ovf + grow;
 #ifdef FR_CAT_TILE_BOUND
       s.m2r = __ldg(p.margin2r + grow); s.er = 0.f; s.bt = 0.f;
@@ -432,9 +433,9 @@ catalog_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       for (int e2 = 0; e2 < sweep_len(sr); ++e2, ++tcount) {
         const uint32_t as = tcount % NACC, aph = (tcount / NACC) & 1u;
         const bool boot = e2 < sr.boot;
-        if (e2 == sr.boot && sr.boot > 0) {             // bootstrap done: K-th largest chunk maximum of every row -> threshold
+        if (e2 == sr.boot && sr.boot > 0) {             // bootstrap done: K_eff-th largest chunk maximum of every row -> threshold
           for (int L = 0; L < 32; ++L) {
-            const CompactOut o = catalog_warp_compact(L, lane, p.cand_sc, p.cand_row, s.base, s.cnt, s.thr, s.m2, p.K, s.ovf, true
+            const CompactOut o = catalog_warp_compact(L, lane, p.cand_sc, p.cand_row, s.base, s.cnt, s.thr, s.m2, s.K, s.ovf, true
                                                       FR_CAT_COMPACT_EXTRA(s, p));
             s.cnt = o.cnt; s.thr = o.thr;
           }

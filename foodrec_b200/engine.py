@@ -42,6 +42,43 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def exclusion_csr(exclude, n):
+    """Per-query-row exclusion lists as a CSR ``(offsets int32 [n+1], ids int32 [nnz])``.
+
+    ``exclude`` is either a tuple ``(offsets, ids)`` (numpy / torch / sequences) or a list of ``n`` per-row sequences
+    of recipe ids.  Host offsets are validated: ``n+1`` entries, the first 0, non-decreasing, the last ``len(ids)``.
+    CUDA tensors are passed through after a length check (validating them would wait for the device).  Ids may be
+    anything in int32: ids the table cannot return are ignored by the kernels."""
+    if isinstance(exclude, tuple):
+        if len(exclude) != 2:
+            raise ValueError("exclude=(offsets, ids) takes two arrays")
+        off, ids = exclude
+        if torch.is_tensor(off) and off.is_cuda and torch.is_tensor(ids) and ids.is_cuda:
+            if off.numel() != n + 1:
+                raise ValueError(f"exclusion offsets: {off.numel()} entries for {n} query rows (want {n + 1})")
+            return off.to(torch.int32).contiguous().reshape(-1), ids.to(torch.int32).contiguous().reshape(-1)
+        off = (off.cpu().numpy() if torch.is_tensor(off) else np.asarray(off)).reshape(-1)
+        ids = (ids.cpu().numpy() if torch.is_tensor(ids) else np.asarray(ids)).reshape(-1)
+    else:
+        rows = [np.asarray(r.cpu().numpy() if torch.is_tensor(r) else r).reshape(-1) for r in exclude]
+        rows = [r if r.size else r.astype(np.int64) for r in rows]          # an empty list is float64 to numpy
+        if len(rows) != n:
+            raise ValueError(f"exclude has {len(rows)} lists for {n} query rows")
+        off = np.zeros(n + 1, np.int64)
+        off[1:] = np.cumsum([r.size for r in rows])
+        ids = np.concatenate(rows) if rows else np.zeros(0, np.int64)
+    if off.size and not np.issubdtype(off.dtype, np.integer) or ids.size and not np.issubdtype(ids.dtype, np.integer):
+        raise TypeError("exclusion offsets and ids must be integers")
+    off = off.astype(np.int64); ids = ids.astype(np.int64)
+    if off.shape != (n + 1,):
+        raise ValueError(f"exclusion offsets: {off.size} entries for {n} query rows (want {n + 1})")
+    if off[0] != 0 or off[-1] != ids.size or (np.diff(off) < 0).any():
+        raise ValueError(f"exclusion offsets must start at 0, be non-decreasing and end at len(ids) = {ids.size}")
+    if ids.size and (ids.min() < -2**31 or ids.max() >= 2**31):
+        raise ValueError("exclusion ids must fit int32")
+    return off.astype(np.int32), ids.astype(np.int32)
+
+
 class Engine:
     def __init__(self, hyper: Hyper, P, R, Cat, G, device="cuda:0", max_rows=1 << 16,
                  max_label_entries=None, adam_mode="lazy", item_cats=None, user_labels=None,
@@ -383,11 +420,15 @@ class Engine:
         L.check(self.handle, self.lib.fr_catalog_prepare(self.handle, C.byref(o), _ptr(self._catalog_cats), self._stream()))
         self._catalog_ready = True
 
-    def catalog_topk(self, users=None, K=100, P_rows=None, n_users=None, id_mul=1, id_add=0, return_scores=True):
+    def catalog_topk(self, users=None, K=100, P_rows=None, n_users=None, id_mul=1, id_add=0, return_scores=True,
+                     exclude=None):
         """The K best recipes of the whole catalog per query user by (score desc, id asc):
         ``ids`` int32 [n,K] (-1 padded), ``scores`` float64 [n,K].  Query rows are
         ``P_rows`` [n,5,D] (device) if given, else ``users`` into Personal_Memory
-        (None = the first ``n_users`` users).  Asynchronous on the current stream."""
+        (None = the first ``n_users`` users).  ``exclude``: recipe ids each query row must not get
+        back (e.g. its training positives), as ``(offsets, ids)`` or a list of per-row sequences
+        (:func:`exclusion_csr`), in the output id space (``local row * id_mul + id_add``).
+        Asynchronous on the current stream."""
         if not getattr(self, "_catalog_ready", False):
             self.catalog_prepare()
         self.flush()
@@ -403,9 +444,17 @@ class Engine:
             n = self.U if n_users is None else int(n_users)
         ids = torch.empty((n, K), dtype=torch.int32, device=self.device)
         sc = torch.empty((n, K), dtype=torch.float64, device=self.device) if return_scores else None
-        L.check(self.handle, self.lib.fr_catalog_topk(self.handle, _ptr(u), _ptr(pr), n, int(K), int(id_mul), int(id_add),
-                                                      _ptr(ids), _ptr(sc), self._stream()))
-        self._keep = [u, pr]
+        if exclude is None:
+            L.check(self.handle, self.lib.fr_catalog_topk(self.handle, _ptr(u), _ptr(pr), n, int(K), int(id_mul), int(id_add),
+                                                          _ptr(ids), _ptr(sc), self._stream()))
+            self._keep = [u, pr]
+        else:
+            off, xi = exclusion_csr(exclude, n)
+            off = self._i32(off)
+            xi = self._i32(xi) if xi.shape[0] else torch.zeros(1, dtype=torch.int32, device=self.device)   # never NULL
+            L.check(self.handle, self.lib.fr_catalog_topk_excluding(self.handle, _ptr(u), _ptr(pr), n, int(K), _ptr(off), _ptr(xi),
+                                                                    int(id_mul), int(id_add), _ptr(ids), _ptr(sc), self._stream()))
+            self._keep = [u, pr, off, xi]
         return (ids, sc) if return_scores else ids
 
     def catalog_merge(self, ids, scores):

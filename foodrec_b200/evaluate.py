@@ -7,6 +7,10 @@ candidate list -- ``[testRatings[u][0]] + testNegatives[u][50:100]`` (``:39-51``
 to the device in one padded [n_users, stride] array and ``fr_eval_sampled_topk`` does
 scoring, dict-dedup and the stable top-K in one launch.  HR / NDCG use the same float64
 ``math.log`` expressions as ``getHitRatio`` / ``getNDCG`` (``:69-81``).
+
+``evaluate_full_catalog`` is the full-ranking protocol (extension): the held-out item is ranked
+against EVERY recipe the user did not train on, through the full-catalog top-K with the user's
+training items excluded.
 """
 from __future__ import annotations
 
@@ -45,4 +49,24 @@ def evaluate_model(sess, model, testRatings, testNegatives, K, dish_to_category)
     rank = rank.cpu().numpy()
     hits = [1 if r >= 0 else 0 for r in rank]                              # getHitRatio :69-73
     ndcgs = [math.log(2) / math.log(int(r) + 2) if r >= 0 else 0 for r in rank]   # getNDCG :76-81
+    return hits, ndcgs
+
+
+def evaluate_full_catalog(sess, model, trainMatrix, testRatings, K, dish_to_category):
+    """Full-ranking HR / NDCG@K per test user, in ``testRatings`` order.  The held-out item is
+    ``testRatings[u][0]`` (``evaluate.py:40``); the candidates are all recipes with a category except
+    the user's training items (``trainMatrix.get(u, [])``, the held-out item itself kept)."""
+    users, held, excl = [], [], {}
+    for user in testRatings:
+        if len(testRatings[str(user)]) == 0:
+            raise ValueError(f"user {user} has no test rating (evaluate.py:37 would return None and crash :29)")
+        h = int(testRatings[str(user)][0])
+        users.append(int(user)); held.append(h)
+        excl[str(int(user))] = [int(i) for i in trainMatrix.get(str(user), []) if int(i) != h]
+    ids, _ = model.catalog_topk(users, K, dish_to_category, exclude=excl)
+    hits, ndcgs = [], []
+    for r, h in enumerate(held):
+        pos = np.nonzero(ids[r] == h)[0]
+        hits.append(1 if pos.size else 0)                                         # getHitRatio :69-73
+        ndcgs.append(math.log(2) / math.log(int(pos[0]) + 2) if pos.size else 0)  # getNDCG :76-81
     return hits, ndcgs

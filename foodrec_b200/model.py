@@ -96,12 +96,13 @@ class Model:
     def score(self, feed):
         return self.engine.score(feed[self.user_input], feed[self.item_input], feed[self.categories])
 
-    def catalog_topk(self, user_ids, K, dish_to_category=None):
+    def catalog_topk(self, user_ids, K, dish_to_category=None, exclude=None):
         """The K best recipes of the WHOLE catalog for each user, by (``model.logits`` desc, id asc) --
         ``evaluate.py:55-63`` with every recipe as a candidate.  ``dish_to_category`` is the reference's
         json map (``Train_recommender.py:132``: item -> [[m0],[m1],[m2],[m3]]); it is only needed on the
-        first call or when it changed.  Returns (ids int32 [n,K], scores float64 [n,K]) as numpy; ids of
-        recipes beyond the catalog are -1."""
+        first call or when it changed.  ``exclude``: a dict keyed like ``Dataset.trainMatrix``
+        (``str(user)`` -> recipe ids) of recipes a user must not get back, e.g. what they trained on.
+        Returns (ids int32 [n,K], scores float64 [n,K]) as numpy; ids of recipes beyond the catalog are -1."""
         e = self.engine
         if dish_to_category is not None:
             ic = np.zeros((e.I, 4), np.float32)
@@ -111,7 +112,8 @@ class Model:
             e.set_item_cats(ic)
         # (the engine rebuilds its recipe index by itself when a training step has run since)
         users = np.asarray([int(u) for u in user_ids], np.int32)
-        ids, sc = e.catalog_topk(users=users, K=int(K))
+        ex = None if exclude is None else [[int(i) for i in exclude.get(str(int(u)), ())] for u in users]
+        ids, sc = e.catalog_topk(users=users, K=int(K), exclude=ex)
         return ids.cpu().numpy(), sc.cpu().numpy()
 
 

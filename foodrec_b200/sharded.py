@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .engine import Engine, Hyper, _ptr
+from .engine import Engine, Hyper, _ptr, exclusion_csr
 
 
 # ---------------------------------------------------------------------------- host-side layout
@@ -308,9 +308,12 @@ class ShardedEngine:
         e._keep = [u]
         return rows
 
-    def catalog_local(self, P_rows_all, K):
-        """Top-K of THIS rank's recipe shard for every gathered query row, ids global."""
-        return self.e.catalog_topk(P_rows=P_rows_all, K=K, id_mul=self.world, id_add=self.rank)
+    def catalog_local(self, P_rows_all, K, exclude=None):
+        """Top-K of THIS rank's recipe shard for every gathered query row, ids global.  ``exclude``: the
+        gathered rows' lists of GLOBAL recipe ids; ids of other shards are ignored by the kernels."""
+        if exclude is None:
+            return self.e.catalog_topk(P_rows=P_rows_all, K=K, id_mul=self.world, id_add=self.rank)
+        return self.e.catalog_topk(P_rows=P_rows_all, K=K, id_mul=self.world, id_add=self.rank, exclude=exclude)
 
     def catalog_merge(self, ids, scores):
         return self.e.catalog_merge(ids, scores)
@@ -430,21 +433,52 @@ class DistRunner:
         return out
 
 
-    def catalog_topk(self, users_local, K=100):
+    def catalog_topk(self, users_local, K=100, exclude=None):
         """Item-sharded full-catalog top-K for this rank's ``users_local`` (same count on every rank):
         all-gather of the query rows, local top-K per recipe shard, all-to-all of the (id, score)
-        lists back to the user owners, exact merge.  Returns ids int32 [n,K], scores float64 [n,K]."""
+        lists back to the user owners, exact merge.  Returns ids int32 [n,K], scores float64 [n,K].
+        ``exclude``: per-user lists of global recipe ids to leave out (``Engine.catalog_topk``); they
+        travel with the query rows (all-gather of the list lengths, then of the ids padded to the
+        longest rank's total)."""
         d, g = self.dist, self.eng
         W = g.world
         rows = g.catalog_query_rows(users_local)
         n = rows.shape[0]
         allrows = torch.empty((W * n,) + tuple(rows.shape[1:]), dtype=rows.dtype, device=rows.device)
         d.all_gather_into_tensor(allrows, rows)
-        ids, sc = g.catalog_local(allrows, K)                 # [W*n, K]: block s = users of rank s
+        if exclude is None:
+            ids, sc = g.catalog_local(allrows, K)             # [W*n, K]: block s = users of rank s
+        else:
+            ids, sc = g.catalog_local(allrows, K, exclude=self._gather_exclusion(exclude, n, rows.device))
         rid, rsc = torch.empty_like(ids), torch.empty_like(sc)
         d.all_to_all_single(rid, ids)                         # block w <- rank w's list for MY users
         d.all_to_all_single(rsc, sc)
         return g.catalog_merge(rid.view(W, n, K), rsc.view(W, n, K))
+
+
+    def _gather_exclusion(self, exclude, n, dev):
+        """This rank's lists for its n query rows -> the CSR of all W*n gathered rows (rank order)."""
+        d, W = self.dist, self.eng.world
+        off, ids = (torch.as_tensor(x).to(dev) for x in exclusion_csr(exclude, n))
+        lens = (off[1:] - off[:-1]).to(torch.int32).contiguous()
+        all_lens = torch.empty(W * n, dtype=torch.int32, device=dev)
+        d.all_gather_into_tensor(all_lens, lens)
+        per_rank = all_lens.view(W, n).sum(1).cpu()
+        m = max(int(per_rank.max()), 1)
+        pad = torch.zeros(m, dtype=torch.int32, device=dev)
+        pad[:ids.numel()] = ids
+        all_ids = torch.empty(W * m, dtype=torch.int32, device=dev)
+        d.all_gather_into_tensor(all_ids, pad)
+        return concat_csr([all_lens[s * n:(s + 1) * n] for s in range(W)],
+                          [all_ids[s * m:s * m + int(per_rank[s])] for s in range(W)])
+
+
+def concat_csr(lens, ids):
+    """CSR (offsets [sum n_s + 1], ids) of the row blocks s = (row lengths lens[s], ids[s]) stacked in order."""
+    lens = torch.cat(lens).to(torch.int64)
+    off = torch.zeros(lens.numel() + 1, dtype=torch.int32, device=lens.device)
+    off[1:] = torch.cumsum(lens, 0).to(torch.int32)
+    return off, torch.cat(ids).to(torch.int32)
 
 
 class LocalRunner:
@@ -510,14 +544,20 @@ class LocalRunner:
         if not p2p: self._all_to_all("grows", "rgrows")
         self._outs = [g.apply() for g in self.engs]
 
-    def catalog_topk(self, users_local_per_rank, K=100):
-        """Same protocol as DistRunner.catalog_topk with the collectives as tensor shuffles."""
+    def catalog_topk(self, users_local_per_rank, K=100, exclude=None):
+        """Same protocol as DistRunner.catalog_topk with the collectives as tensor shuffles.  ``exclude``:
+        one entry per rank, that rank's per-user lists of global recipe ids (or None)."""
         W = self.W
         rows = [g.catalog_query_rows(u) for g, u in zip(self.engs, users_local_per_rank)]
         n = rows[0].shape[0]
         assert all(r.shape[0] == n for r in rows)
         allrows = torch.cat(rows, 0)
-        lists = [g.catalog_local(allrows, K) for g in self.engs]          # per recipe shard: [W*n, K]
+        if exclude is None:
+            lists = [g.catalog_local(allrows, K) for g in self.engs]      # per recipe shard: [W*n, K]
+        else:
+            csr = [tuple(torch.as_tensor(x) for x in exclusion_csr(ex, n)) for ex in exclude]
+            ex = concat_csr([off[1:] - off[:-1] for off, _ in csr], [ids for _, ids in csr])
+            lists = [g.catalog_local(allrows, K, exclude=ex) for g in self.engs]
         out = []
         for r, g in enumerate(self.engs):
             ids = torch.stack([lists[w][0][r * n:(r + 1) * n] for w in range(W)])

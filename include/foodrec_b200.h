@@ -284,6 +284,17 @@ int fr_catalog_prepare(fr_handle h, const fr_catalog_opts* opts, const float* it
  * fp64 or NULL.  Asynchronous on the stream. */
 int fr_catalog_topk(fr_handle h, const int32_t* users, const float* P_rows, int32_t n_users, int32_t K,
                     int32_t id_mul, int32_t id_add, int32_t* out_ids, double* out_scores, fr_stream s);
+/* fr_catalog_topk that leaves out, per query row, the recipes the caller lists (e.g. the user's training positives):
+ * the K best by (score desc, id asc) among the recipes that have a category and are NOT on the row's list, -1 / -inf
+ * padded when fewer remain.  Lists are a CSR over query rows on the device: excl_off [n_users+1], excl_ids [nnz]
+ * (int32; both NULL = no lists = fr_catalog_topk, bit for bit).  Ids are in the OUTPUT id space (local row * id_mul
+ * + id_add), so a recipe shard takes the global lists unchanged; any order, duplicates allowed; an id this table
+ * cannot return (another shard's, out of range, negative) is ignored.  The filter is widened per row by the row's
+ * listed recipes of this table (csrc/catalog.cuh); a row with K + that count > 256 takes the exact fallback
+ * (counted by fr_catalog_fallback_rows).  id_mul >= 1 with lists.  Asynchronous on the stream. */
+int fr_catalog_topk_excluding(fr_handle h, const int32_t* users, const float* P_rows, int32_t n_users, int32_t K,
+                              const int32_t* excl_off, const int32_t* excl_ids, int32_t id_mul, int32_t id_add,
+                              int32_t* out_ids, double* out_scores, fr_stream s);
 /* Dense copies of Personal_Memory rows: out[k] = P[users[k]] ([n,5,D], device) -- the query rows a rank contributes to
  * the all-gather of the item-sharded top-K (a user id outside the table yields a zero row). */
 int fr_gather_user_rows(fr_handle h, const int32_t* users, int32_t n, float* out, fr_stream s);
