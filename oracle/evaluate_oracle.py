@@ -52,10 +52,44 @@ def evaluate_model(model, testRatings, testNegatives, K, item_cats):
     return hits, ndcgs, ranks
 
 
-def catalog_topk(model, users, item_cats, K, dtype=np.float64):
-    """Full-catalog scoring (extension; definition = ``inference`` over every
-    recipe).  Scores in ``dtype`` from the model's tables; top-K by
-    (score desc, id asc)."""
+def sampled_topk(scores, cand, n_cand, K, valid_user=None):
+    """``eval_one_rating``'s ranking (dict of the candidates, later score wins,
+    first position kept; ``heapq.nlargest``: score desc, ties in insertion
+    order), vectorised over many users.  ``scores[r, j]`` is candidate j's score
+    for row r.  Candidates past ``n_cand[r]`` and ids < 0 are not in the list.
+    Returns top-K ids [n, K] padded with -1 and the rank of candidate 0's id in
+    them (-1: not among them); rows with ``valid_user`` False get no list."""
+    scores = np.asarray(scores, np.float64); cand = np.asarray(cand, np.int64)
+    n, stride = cand.shape
+    j = np.arange(stride)
+    live = (j[None, :] < np.asarray(n_cand)[:, None]) & (cand >= 0)
+    if valid_user is not None:
+        live &= np.asarray(valid_user, bool)[:, None]
+    r, p = np.nonzero(live)                      # row-major: positions ascending within a row
+    c, s = cand[r, p], scores[r, p]
+    # dict semantics: group equal (row, id); the first position survives with the last position's score
+    o = np.lexsort((p, c, r))
+    r, p, c, s = r[o], p[o], c[o], s[o]
+    head = np.ones(len(r), bool); head[1:] = (r[1:] != r[:-1]) | (c[1:] != c[:-1])
+    tail = np.ones(len(r), bool); tail[:-1] = head[1:]
+    r, p, c, s = r[head], p[head], c[head], s[tail]
+    # nlargest: score desc, then position asc
+    o = np.lexsort((p, -s, r))
+    r, c = r[o], c[o]
+    start = np.searchsorted(r, np.arange(n))
+    k = np.arange(len(r)) - start[r]
+    ids = np.full((n, K), -1, np.int64)
+    keep = k < K
+    ids[r[keep], k[keep]] = c[keep]
+    gt = np.where(live[:, 0], cand[:, 0], -1)
+    hit = (ids == gt[:, None]) & (gt[:, None] >= 0)
+    rank = np.where(hit.any(1), hit.argmax(1), -1)
+    return ids, rank
+
+
+def catalog_scores(model, users, item_cats, dtype=np.float64):
+    """Score of every (user, recipe) pair, [len(users), I], by the GEMM form of
+    ``inference`` (SURVEY App. A.1) in ``dtype``."""
     P = model.P.astype(dtype); R = model.R.astype(dtype); Cat = model.Cat.astype(dtype)
     cats = item_cats.astype(dtype)
     n = cats.sum(1, keepdims=True)
@@ -67,7 +101,15 @@ def catalog_topk(model, users, item_cats, K, dtype=np.float64):
     for c in range(4):
         Q[:, (1 + c) * D:(2 + c) * D] = b * w[:, c:c + 1] * R
     users = np.asarray(users, np.int64)
-    S = P[users].reshape(len(users), 5 * D) @ Q.T
+    return P[users].reshape(len(users), 5 * D) @ Q.T
+
+
+def catalog_topk(model, users, item_cats, K, dtype=np.float64):
+    """Full-catalog scoring (extension; definition = ``inference`` over every
+    recipe).  Scores in ``dtype`` from the model's tables; top-K by
+    (score desc, id asc)."""
+    S = catalog_scores(model, users, item_cats, dtype)
+    I = S.shape[1]
     ids = np.empty((len(users), K), np.int64)
     sc = np.empty((len(users), K), dtype)
     ar = np.arange(I)

@@ -67,7 +67,7 @@ def test_radix_sort_is_stable_and_exact(n, nbits):
 
 
 # ---------------------------------------------------------------- forward
-@pytest.mark.parametrize("D", [16, 64, 128, 200])
+@pytest.mark.parametrize("D", [4, 16, 64, 128, 132, 200, 256])
 def test_fwd_score_matches_oracle(D):
     p = Problem(300, 200, 7, D, seed=D)
     e = make_engine(p)
@@ -90,7 +90,7 @@ def test_fwd_score_general_float_category_weights():
 # ---------------------------------------------------------------- train step
 @pytest.mark.parametrize("learner,adam_mode", [("sgd", "dense"), ("adagrad", "dense"), ("rmsprop", "dense"),
                                                ("adam", "dense"), ("adam", "lazy_exact"), ("adam", "lazy")])
-@pytest.mark.parametrize("D", [64, 200])
+@pytest.mark.parametrize("D", [4, 64, 132, 200, 256])
 def test_pointwise_steps_match_oracle(learner, adam_mode, D):
     p = Problem(500, 300, 9, D, seed=17)
     e = make_engine(p, learner=learner, adam_mode=adam_mode)

@@ -54,16 +54,26 @@ def gather(engs, p):
     ("adam", "lazy", True, False), ("adam", "lazy_exact", False, False)])
 def test_sharded_equals_unsharded(W, learner, adam_mode, bpr, single_pass):
     p = Problem(403, 257, 9, 64, seed=61)            # sizes not divisible by W: padded shards
-    single, engs = build(p, W, learner, adam_mode, single_pass=single_pass)
+    # W = 2 adds a step whose rows are ~90 % one recipe: each rank's recipe-gradient pre-reduction then holds a run of
+    # more than 16 chunks of 32 rows, which seg_combine_long_kernel sums (ItemGradPol, peer or local stores)
+    hot = W == 2
+    single, engs = build(p, W, learner, adam_mode, max_rows=4096 if hot else 2048, single_pass=single_pass)
     if learner == "adam" and adam_mode != "dense":
         assert all(g.e.single_pass == (single_pass is None) for g in engs)
     run = sharded.LocalRunner(engs)
-    for s in range(5):
-        B = 300
+    for s in range(6 if hot else 5):
+        B = 1400 if s == 5 else 300
         users = None
         if s == 2:
             users = np.repeat(np.arange(12), 25)      # duplicate-heavy, runs cross chunks
         f = p.bpr(B, seed=80 + s, users=users) if bpr else p.pointwise(B, seed=80 + s, users=users)
+        if s == 5:
+            rng = np.random.default_rng(s)
+            it = np.where(rng.random(B) < 0.9, 5, f["item_input"]).astype(np.int32)
+            f["item_input"], f["categories"] = it, p.item_cats[it].reshape(B, 4, 1).copy()
+            if bpr:
+                f["neg_item_input"] = np.where(f["neg_item_input"] == it, (it + 1) % p.I, f["neg_item_input"]).astype(np.int32)
+                f["neg_categories"] = p.item_cats[f["neg_item_input"]].reshape(B, 4, 1).copy()
         personal = (s == 0)
         # unsharded reference: compact feed so both sides use the same side tables
         kw = dict(neg_items=f["neg_item_input"], neg_categories=f["neg_categories"]) if bpr else {}

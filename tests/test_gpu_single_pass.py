@@ -39,7 +39,8 @@ def feeds(p, bpr, n, seed, B=700):
 
 
 @pytest.mark.parametrize("bpr", [False, True])
-@pytest.mark.parametrize("D,adam_mode", [(64, "lazy"), (128, "lazy"), (128, "lazy_exact"), (200, "lazy")])
+@pytest.mark.parametrize("D,adam_mode", [(4, "lazy"), (64, "lazy"), (128, "lazy"), (128, "lazy_exact"), (132, "lazy"),
+                                       (200, "lazy"), (256, "lazy_exact")])
 def test_single_pass_equals_two_pass_and_oracle(bpr, D, adam_mode):
     p = Problem(900, 500, 9, D, seed=3 + D)
     a, b = engine(p, True, adam_mode), engine(p, False, adam_mode)

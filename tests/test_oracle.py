@@ -151,6 +151,40 @@ def test_evaluate_restatement_semantics():
     assert rl == [6, 7, 5] and hr == 1 and ndcg == pytest.approx(np.log(2) / np.log(4))
 
 
+@pytest.mark.parametrize("K", [1, 3, 10, 60])
+def test_vectorised_sampled_ranking_equals_eval_one_rating(K):
+    """evaluate_oracle.sampled_topk (all users at once) against the per-user dict + heapq.nlargest of evaluate.py on
+    lists drawn from 12 ids (repeats within a list, of the positive too) with integer scores per POSITION (exact ties,
+    and a repeated id whose later occurrence carries a different score)."""
+    rng = np.random.default_rng(K)
+    n, stride = 400, 51
+    cand = rng.integers(0, 12, (n, stride))
+    n_cand = rng.integers(1, stride + 1, n)
+    n_cand[:4] = [1, 2, 32, 33]
+    scores = rng.integers(-3, 4, (n, stride)).astype(np.float64)
+
+    class Fake:
+        row = 0
+
+        def scores(self, u, it, cats):
+            return scores[self.row, :len(it)]
+    fake = Fake()
+    ids, rank = evaluate_oracle.sampled_topk(scores, cand, n_cand, K)
+    for r in range(n):
+        tr = {"0": [int(cand[r, 0])]}
+        tn = {"0": [0] * 50 + cand[r, 1:n_cand[r]].tolist()}
+        fake.row = r
+        _, _, rl = evaluate_oracle.eval_one_rating(fake, "0", tr, tn, K, np.zeros((12, 4)))
+        assert ids[r][ids[r] >= 0].tolist() == rl, r
+        assert rank[r] == (rl.index(cand[r, 0]) if cand[r, 0] in rl else -1), r
+    # ids < 0, positions past n_cand and rows of users outside the table are not ranked
+    c2 = cand.copy(); c2[:, 0] = -1
+    valid = np.arange(n) % 7 != 0
+    ids2, rank2 = evaluate_oracle.sampled_topk(scores, c2, n_cand, K, valid_user=valid)
+    assert (ids2[~valid] == -1).all() and (rank2 == -1).all()
+    assert not np.isin(ids2[valid & (n_cand == 1)], np.arange(12)).any()
+
+
 def test_get_train_instances_shape():
     p = Problem(12, 400, 5, 4, seed=8)
     train, tr, tn = synth.make_reference_dataset(12, 400, seed=1, pos_range=(3, 9))
