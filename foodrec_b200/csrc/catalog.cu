@@ -38,6 +38,7 @@ struct CatalogWs {
   int mp_cap = 0;
   __nv_bfloat16* A = nullptr; float *bias = nullptr, *margin2 = nullptr, *cand_sc = nullptr;
   int32_t *cand_row = nullptr, *cand_cnt = nullptr, *ovf = nullptr, *ovf_list = nullptr, *ovf_count = nullptr, *keff = nullptr;
+  int32_t* call_ovf = nullptr;            // rows of the current call (all passes) that took the exact fallback
   double* scratch = nullptr; int exact_blocks = 0;
   unsigned long long* dbg = nullptr;
   uint32_t* ukeys = nullptr; SortBufs sortU; int32_t* block_first = nullptr;   // users sorted by best mask group
@@ -368,7 +369,8 @@ struct FinParams {
 #ifdef FR_CAT_TILE_BOUND
   const float* margin2r; const float* tile_rho; int bn_shift;
 #endif
-  const int32_t* ovf; int32_t* ovf_list; int32_t* ovf_count;
+  const int32_t* ovf; int32_t* ovf_list; int32_t* ovf_count;   // ovf_count: this pass's fallback rows (the fallback's work list)
+  int32_t* call_ovf;                        // the call's fallback rows over all passes (fr_catalog_fallback_rows)
   const int32_t* keff;                      // [m_pad] per-row K_eff
   ExclLists excl;                           // carries id_mul / id_add of the outputs too
   int id_mul, id_add;
@@ -478,7 +480,7 @@ __global__ void __launch_bounds__(FIN_THREADS) cat_finalize_kernel(const FinPara
     }
   }
   if (overflow) {                       // exact fallback takes this row
-    if (tid == 0) { const int slot = atomicAdd(f.ovf_count, 1); f.ovf_list[slot] = row; }
+    if (tid == 0) { const int slot = atomicAdd(f.ovf_count, 1); f.ovf_list[slot] = row; atomicAdd(f.call_ovf, 1); }
     return;
   }
   const int nF = s_nF;
@@ -854,33 +856,54 @@ extern "C" int fr_catalog_prepare(fr_handle h, const fr_catalog_opts* opts, cons
   return FR_OK;
 }
 
-static int catalog_ensure_pass_ws(fr_ctx* h, CatalogWs& w, int mp) {
+// (Re)allocation of a pass buffer: the buffer it had is freed first (cudaFree waits for the device).
+static void pass_free(fr_ctx* h, void* p) {
+  if (p) for (auto& q : h->allocs) if (q == p) { cudaFree(q); q = nullptr; }
+}
+template <class T>
+static int pass_alloc(fr_ctx* h, T** p, size_t n) {
+  pass_free(h, *p);
+  *p = nullptr;
+  return dalloc(h, p, n);
+}
+
+// Pass workspace for passes of up to mp rows.  A later call that needs more rows than it has (a re-prepare with a
+// larger max_pass_rows, or the defaults after a small one) replaces the row-sized buffers once the stream is idle.
+static int catalog_ensure_pass_ws(fr_ctx* h, CatalogWs& w, int mp, cudaStream_t st) {
   if (mp <= w.mp_cap) return FR_OK;
-  if (w.mp_cap != 0) return fail(h, FR_ERR_STATE, "catalog pass workspace was sized for %d rows", w.mp_cap);
+  if (w.mp_cap != 0) FR_CUDA(h, cudaStreamSynchronize(st));
+  w.mp_cap = 0;                     // until every buffer below has its new size
   int rc;
   const size_t R = (size_t)mp;
-  if ((rc = dalloc(h, &w.A, 16 * R * w.KP * 2))) return rc;
-  if ((rc = dalloc(h, &w.bias, 16 * R))) return rc;
-  if ((rc = dalloc(h, &w.margin2, R))) return rc;
+  if ((rc = pass_alloc(h, &w.A, 16 * R * w.KP * 2))) return rc;
+  if ((rc = pass_alloc(h, &w.bias, 16 * R))) return rc;
+  if ((rc = pass_alloc(h, &w.margin2, R))) return rc;
 #ifdef FR_CAT_TILE_BOUND
-  if ((rc = dalloc(h, &w.margin2r, R))) return rc;
+  if ((rc = pass_alloc(h, &w.margin2r, R))) return rc;
 #endif
   const size_t RL = R * 4;          // candidate lists: up to 4 column sets per (split, row)
-  if ((rc = dalloc(h, &w.cand_sc, RL * CAT_CAP))) return rc;
-  if ((rc = dalloc(h, &w.cand_row, RL * CAT_CAP))) return rc;
-  if ((rc = dalloc(h, &w.cand_cnt, RL))) return rc;
-  if ((rc = dalloc(h, &w.ovf, R))) return rc;
-  if ((rc = dalloc(h, &w.keff, R))) return rc;
-  if ((rc = dalloc(h, &w.ovf_list, R))) return rc;
-  if ((rc = dalloc(h, &w.ovf_count, 1))) return rc;
-  if ((rc = dalloc(h, &w.dbg, 8))) return rc;
-  FR_CUDA(h, cudaMemset(w.dbg, 0, 64));
-  if ((rc = dalloc(h, &w.ukeys, R))) return rc;
+  if ((rc = pass_alloc(h, &w.cand_sc, RL * CAT_CAP))) return rc;
+  if ((rc = pass_alloc(h, &w.cand_row, RL * CAT_CAP))) return rc;
+  if ((rc = pass_alloc(h, &w.cand_cnt, RL))) return rc;
+  if ((rc = pass_alloc(h, &w.ovf, R))) return rc;
+  if ((rc = pass_alloc(h, &w.keff, R))) return rc;
+  if ((rc = pass_alloc(h, &w.ovf_list, R))) return rc;
+  if ((rc = pass_alloc(h, &w.ukeys, R))) return rc;
+  for (void* p : {(void*)w.sortU.k[0], (void*)w.sortU.k[1], (void*)w.sortU.v[0], (void*)w.sortU.v[1], (void*)w.sortU.tile_hist,
+                  (void*)w.sortU.ticket, (void*)w.sortU.scan_tmp})
+    pass_free(h, p);
+  w.sortU = SortBufs();
   if ((rc = alloc_sort(h, w.sortU, R))) return rc;
-  if ((rc = dalloc(h, &w.block_first, R / CAT_BM + 1))) return rc;
-  const size_t budget = (size_t)512 << 20;
-  w.exact_blocks = (int)std::max<size_t>(2, std::min<size_t>((size_t)h->sm_count, budget / ((size_t)w.I * 8)));
-  if ((rc = dalloc(h, &w.scratch, (size_t)w.exact_blocks * w.I))) return rc;
+  if ((rc = pass_alloc(h, &w.block_first, R / CAT_BM + 1))) return rc;
+  if (!w.scratch) {                 // sized by the catalog, not by the pass
+    if ((rc = dalloc(h, &w.ovf_count, 1))) return rc;
+    if ((rc = dalloc(h, &w.call_ovf, 1))) return rc;
+    if ((rc = dalloc(h, &w.dbg, 8))) return rc;
+    FR_CUDA(h, cudaMemset(w.dbg, 0, 64));
+    const size_t budget = (size_t)512 << 20;
+    w.exact_blocks = (int)std::max<size_t>(2, std::min<size_t>((size_t)h->sm_count, budget / ((size_t)w.I * 8)));
+    if ((rc = dalloc(h, &w.scratch, (size_t)w.exact_blocks * w.I))) return rc;
+  }
   w.mp_cap = mp;
   return FR_OK;
 }
@@ -907,8 +930,9 @@ extern "C" int fr_catalog_topk_excluding(fr_handle h, const int32_t* users, cons
   // rows per pass: whole waves of user blocks; small calls split the recipe sweep instead
   const int pass_rows = w.max_pass_rows > 0 ? (w.max_pass_rows + BMC - 1) / BMC * BMC : n_clusters * BMC * 4;
   const int NSET = w.epi_sets;
-  int rc = catalog_ensure_pass_ws(h, w, std::max(pass_rows, 2 * n_clusters * BMC));
+  int rc = catalog_ensure_pass_ws(h, w, std::max(pass_rows, 2 * n_clusters * BMC), st);
   if (rc) return rc;
+  FR_CUDA(h, cudaMemsetAsync(w.call_ovf, 0, 4, st));
   const int D = h->mc.D, DV = h->mc.DV;
   // |s_hat - s| <= cfac * |A||R|.  bf16 rounding u = 2^-8 on both operands: 2u + u^2; with the split
   // user operand (exact to 2^-16) only the recipe side rounds: u + 2^-15.  Plus fp32 accumulation.
@@ -1000,7 +1024,7 @@ extern "C" int fr_catalog_topk_excluding(fr_handle h, const int32_t* users, cons
 #ifdef FR_CAT_TILE_BOUND
     f.margin2r = w.margin2r; f.tile_rho = w.tile_rho; f.bn_shift = w.BN == 256 ? 8 : 7;
 #endif
-    f.ovf = w.ovf; f.ovf_list = w.ovf_list; f.ovf_count = w.ovf_count; f.keff = w.keff; f.excl = excl;
+    f.ovf = w.ovf; f.ovf_list = w.ovf_list; f.ovf_count = w.ovf_count; f.call_ovf = w.call_ovf; f.keff = w.keff; f.excl = excl;
     f.id_mul = id_mul; f.id_add = id_add; f.out_ids = out_ids; f.out_scores = out_scores;
     const size_t fsm = (size_t)CAT_FCAP * (8 + 4 + 4) + 32 + (size_t)5 * D * 4 + (size_t)n_lists * CAT_CAP * 8 +
                        (size_t)16 * D * 8 + 8;      // + the per-mask fp64 user rows of the re-rank
@@ -1072,9 +1096,9 @@ extern "C" int fr_catalog_timing_read(fr_handle h, double* ms_sum, int64_t* n_pa
 
 extern "C" int fr_catalog_fallback_rows(fr_handle h, int32_t* out, fr_stream s) {
   if (!h || !out) return FR_ERR_ARG;
-  if (!h->cat || !h->cat->ovf_count) return fail(h, FR_ERR_STATE, "no catalog pass has run");
+  if (!h->cat || !h->cat->call_ovf) return fail(h, FR_ERR_STATE, "no catalog pass has run");
   cudaStream_t st = static_cast<cudaStream_t>(s);
-  FR_CUDA(h, cudaMemcpyAsync(out, h->cat->ovf_count, 4, cudaMemcpyDeviceToHost, st));
+  FR_CUDA(h, cudaMemcpyAsync(out, h->cat->call_ovf, 4, cudaMemcpyDeviceToHost, st));
   FR_CUDA(h, cudaStreamSynchronize(st));
   return FR_OK;
 }

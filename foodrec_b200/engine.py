@@ -402,22 +402,33 @@ class Engine:
         self.item_cats = ic
         self._set_tables()
         self._catalog_ready = False
+        self._catalog_cats_given = None             # a map passed to catalog_prepare was derived from the old one
 
     # ------------------------------------------------------------------ full-catalog top-K
     def catalog_prepare(self, cta_group=0, max_pass_rows=0, splits=0, epi_sets=0, tile_n=0, a_split=0, item_cats=None):
         """Build the recipe-side index of the catalog kernel from the current R / item_cats
         (call again after training changed R).  ``item_cats`` [I,4]: the masks of THIS table's
-        rows when the resident table is a global map (row-sharded engines).  Synchronises."""
+        rows when the resident table is a global map (a ``ShardedEngine`` sets its slice as the
+        default).  The arguments are kept: when training has made the index stale,
+        ``catalog_topk`` rebuilds it with the same ones.  Synchronises."""
+        cats = None
         if item_cats is not None:
-            self._catalog_cats = torch.as_tensor(np.asarray(item_cats, np.float32).reshape(-1, 4)).to(self.device).contiguous()
-            assert self._catalog_cats.shape[0] == self.I
-        elif self.item_cats is None:
+            cats = torch.as_tensor(np.asarray(item_cats, np.float32).reshape(-1, 4)).to(self.device).contiguous()
+            assert cats.shape[0] == self.I
+        self._catalog_cats_given = cats
+        self._catalog_opts = L.fr_catalog_opts(int(cta_group), int(max_pass_rows), int(splits), int(epi_sets), int(tile_n),
+                                               int(a_split))
+        self._catalog_build()
+
+    def _catalog_build(self):
+        cats = self._catalog_cats_given
+        if cats is None:
+            cats = getattr(self, "_catalog_local_cats", None)
+        if cats is None and self.item_cats is None:
             raise L.FoodRecError("catalog scoring needs the item_cats (dish_to_category) table")
-        else:
-            self._catalog_cats = None
+        self._catalog_cats = cats                # (the library keeps the pointer: held as long as the index)
         self.flush()
-        o = L.fr_catalog_opts(int(cta_group), int(max_pass_rows), int(splits), int(epi_sets), int(tile_n), int(a_split))
-        L.check(self.handle, self.lib.fr_catalog_prepare(self.handle, C.byref(o), _ptr(self._catalog_cats), self._stream()))
+        L.check(self.handle, self.lib.fr_catalog_prepare(self.handle, C.byref(self._catalog_opts), _ptr(cats), self._stream()))
         self._catalog_ready = True
 
     def catalog_topk(self, users=None, K=100, P_rows=None, n_users=None, id_mul=1, id_add=0, return_scores=True,
@@ -430,7 +441,10 @@ class Engine:
         (:func:`exclusion_csr`), in the output id space (``local row * id_mul + id_add``).
         Asynchronous on the current stream."""
         if not getattr(self, "_catalog_ready", False):
-            self.catalog_prepare()
+            if getattr(self, "_catalog_opts", None) is None:
+                self.catalog_prepare()
+            else:
+                self._catalog_build()          # stale index: rebuilt with the options and masks it was prepared with
         self.flush()
         pr = u = None
         if P_rows is not None:

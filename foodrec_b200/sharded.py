@@ -81,6 +81,11 @@ class ShardedEngine:
         e = self.e
         self.device = e.device
         self.I_global = None if item_cats_global is None else int(len(item_cats_global))
+        if item_cats_global is not None:
+            # the catalog index of this rank's recipe shard reads the masks of ITS rows (local row k = recipe
+            # rank + k*W), never the first rows of the global map: every (re)build of the index uses this slice
+            e._catalog_local_cats = torch.as_tensor(
+                shard_rows(np.asarray(item_cats_global, np.float32).reshape(-1, 4), rank, world)).to(e.device).contiguous()
         if cap is None:
             # unique recipes per (source, owner).  A batch has at most max_rows distinct recipes,
             # spread over the owners by id % W: max_rows/W on average even when every row is
@@ -292,11 +297,9 @@ class ShardedEngine:
     def catalog_prepare(self, **opts):
         """Index of THIS rank's recipe shard (local row k = recipe rank + k*W; rows past the
         catalog end carry no category and are never returned)."""
-        e = self.e
-        cats = e.item_cats.cpu().numpy() if e.item_cats is not None else None
-        if cats is None:
+        if getattr(self.e, "_catalog_local_cats", None) is None:
             raise L.FoodRecError("catalog scoring needs the global item_cats map")
-        e.catalog_prepare(item_cats=shard_rows(cats, self.rank, self.world), **opts)
+        self.e.catalog_prepare(**opts)
 
     def catalog_query_rows(self, users_local):
         """This rank's query users as dense [n,5,D] rows (what the all-gather moves)."""

@@ -264,7 +264,9 @@ int fr_shard_apply(fr_handle h, const fr_shard* sh, const int32_t* rreq, const f
  *
  * fr_catalog_prepare builds the recipe-side index from the CURRENT R / item_cats (recipes
  * grouped by category mask, bf16 operand, norms).  It synchronises the stream and must be
- * called again after R or item_cats change.  P and Cat are read at query time. */
+ * called again after R or item_cats change.  P and Cat are read at query time.  A query whose
+ * passes need more workspace than earlier queries allocated (e.g. after a re-prepare with a larger
+ * max_pass_rows) re-allocates it, synchronising its stream first. */
 typedef struct {
   int32_t cta_group;      /* 0 = default (2: CTA pairs, tcgen05 cta_group::2), 1 = single-CTA MMA */
   int32_t max_pass_rows;  /* 0 = default; users processed per pass */
@@ -311,7 +313,9 @@ int fr_catalog_info(fr_handle h, int32_t* out /* [8] */);
  * FOODREC_CATALOG_CYCLES is set): {MMA thread total, waiting for a free accumulator, waiting for
  * operands, #MMA threads, epilogue warp total, waiting for an accumulator, #epilogue warps, 0}; resets. */
 int fr_catalog_cycle_counters(fr_handle h, uint64_t* out /* [8] */, fr_stream s);
-/* rows of the LAST pass that took the exact full-scan fallback (synchronises the stream) */
+/* rows of the LAST fr_catalog_topk / fr_catalog_topk_excluding call, all of its passes, that took the exact
+ * full-scan fallback: rows flagged up front (K + listed recipes > 256) and rows whose candidates overflowed
+ * (synchronises the stream) */
 int fr_catalog_fallback_rows(fr_handle h, int32_t* out, fr_stream s);
 
 /* ---- Negative sampling for 1:N BPR (extension; the reference only takes listed negatives,

@@ -46,6 +46,42 @@ def catalog_topk_excluding(model, users, item_cats, K, exclude, dtype=np.float64
     return ids, sc
 
 
+def catalog_topk_chunked(model, users, item_cats, K, exclude=None, chunk=32, dtype=np.float64):
+    """``catalog_topk_excluding`` (``exclude`` None: ``evaluate_oracle.catalog_topk``) for large catalogs: the recipe
+    operand of ``catalog_scores`` is formed once, users are scored ``chunk`` at a time, and each row sorts only a
+    superset of its top-K -- every candidate whose score reaches the K-th largest (all ties with it included)."""
+    P = model.P.astype(dtype); R = model.R.astype(dtype); Cat = model.Cat.astype(dtype)
+    cats = item_cats.astype(dtype)
+    w = cats / cats.sum(1, keepdims=True)
+    a = dtype(model.a); b = dtype(model.one_minus_a)
+    I, D = R.shape
+    Q = np.empty((I, 5 * D), dtype)                  # the operand of catalog_scores
+    Q[:, :D] = a * (w @ Cat)
+    for c in range(4):
+        Q[:, (1 + c) * D:(2 + c) * D] = b * w[:, c:c + 1] * R
+    users = np.asarray(users, np.int64)
+    n = len(users)
+    ids = np.full((n, K), -1, np.int64)
+    sc = np.full((n, K), -np.inf, dtype)
+    for r0 in range(0, n, chunk):
+        S = P[users[r0:r0 + chunk]].reshape(-1, 5 * D) @ Q.T
+        for j in range(S.shape[0]):
+            r = r0 + j
+            keep = np.ones(I, bool)
+            if exclude is not None:
+                ex = np.asarray(exclude[r], np.int64).reshape(-1)
+                keep[ex[(ex >= 0) & (ex < I)]] = False
+            k = min(K, int(keep.sum()))
+            if k == 0:
+                continue
+            s = np.where(keep, S[j], -np.inf)
+            kth = s[np.argpartition(-s, k - 1)[k - 1]]
+            cand = np.nonzero(keep & (s >= kth))[0]
+            order = cand[np.lexsort((cand, -s[cand]))][:k]
+            ids[r, :k], sc[r, :k] = order, S[j, order]
+    return ids, sc
+
+
 def evaluate_full_catalog(model, trainMatrix, testRatings, K, item_cats):
     """Full-ranking HR / NDCG@K per test user (``testRatings`` order); scores in float64, recipes without a category
     never ranked (the catalog path does not return them)."""

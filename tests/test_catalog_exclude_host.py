@@ -137,6 +137,30 @@ def test_oracle_excluding_the_true_topk_gives_ranks_k1_to_2k():
     assert np.array_equal(ids, full[:, K:]) and np.array_equal(sc, fsc[:, K:])
 
 
+@pytest.mark.parametrize("chunk", [1, 4, 32])
+def test_chunked_oracle_equals_the_full_sort(chunk):
+    """catalog_topk_chunked (partial selection, users in chunks) == the full lexsort of catalog_topk_excluding and
+    evaluate_oracle.catalog_topk: lists, padding, and rows where every score ties (all-zero user rows).  Ids exactly;
+    scores to the last bits (BLAS may sum a chunk's product in another order than the whole batch's)."""
+    def same(a, b):
+        assert np.array_equal(a[0], b[0]) and np.array_equal(np.isfinite(a[1]), np.isfinite(b[1]))
+        f = np.isfinite(b[1])
+        assert np.abs(a[1][f] - b[1][f]).max() <= 1e-14 * np.abs(b[1][f]).max()
+
+    U, I, D, K = 12, 700, 16, 30
+    om, ic = _oracle(U, I, D, seed=5)
+    om.P[4] = 0                                                      # 700-way tie: lowest ids first
+    om.P[9, 1:] = 0                                                  # ties within each category mask
+    rng = np.random.default_rng(3)
+    users = np.array([0, 3, 3, 11, 7, 5, 4, 9, 4, 9])
+    excl = [[], list(range(I - 10)), list(range(I)), list(rng.integers(0, I, 40)) * 2 + [-1, I, I + 9],
+            [], [], [], [], list(range(0, 60, 2)), list(range(5))]
+    ids, sc = xo.catalog_topk_chunked(om, users, ic, K, excl, chunk=chunk)
+    same((ids, sc), xo.catalog_topk_excluding(om, users, ic, K, excl))
+    assert (ids[1] >= 0).sum() == 10 and (ids[2] == -1).all() and ids[6].tolist() == list(range(K))
+    same(xo.catalog_topk_chunked(om, users, ic, K, chunk=chunk), evaluate_oracle.catalog_topk(om, users, ic, K))
+
+
 def test_oracle_full_catalog_evaluation_on_the_reference_dataset():
     from foodrec_b200.data import Dataset, side_tables
     d = Dataset(os.path.join(GOLD, "ref_dataset", "toy"))
