@@ -15,7 +15,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libfoodrec_b200.so")
-SOURCES = ["sort.cu", "train_fwd.cu", "train_seg.cu", "train_shard.cu", "eval.cu", "catalog.cu", "catalog_gemm.cu", "sampler.cu", "api.cu", "api_shard.cu"]
+SOURCES = ["sort.cu", "train_fwd.cu", "train_seg.cu", "train_shard.cu", "eval.cu", "catalog.cu", "catalog_gemm.cu", "sampler.cu", "api.cu", "api_shard.cu",
+           "eval_shard.cu"]
 HEADERS = ["common.cuh", "internal.h", "train.cuh", "optim.cuh", "ctx.h", "catalog.cuh", "tc05.cuh",
            os.path.join("..", "..", "include", "foodrec_b200.h")]
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

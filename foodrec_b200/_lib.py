@@ -111,6 +111,12 @@ _PROTOS = {
     "fr_shard_update": (C.c_int, [C.c_void_p, C.POINTER(fr_batch), C.POINTER(fr_shard), C.c_int32, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p, C.c_void_p]),
     "fr_shard_apply": (C.c_int, [C.c_void_p, C.POINTER(fr_shard), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_shard_eval_plan": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_shard_eval_serve": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "fr_eval_sampled_rows": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p,
+                                       C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p]),
 }
 
 _lib = None

@@ -78,6 +78,13 @@ struct fr_ctx {
     float4* pieces_s = nullptr;
     fr::PeerPtrs peer_rbuf{}, peer_rgrows{};   // fr_shard_set_peers: NVLink P2P exchange instead of all-to-alls
   } sh;
+  // sampled evaluation on row-sharded tables (eval_shard.cu): workspace of fr_shard_eval_plan for n_cap candidate
+  // entries, re-allocated (after a stream synchronise) when a call needs more
+  struct EvalPlanWs {
+    size_t n_cap = 0;
+    uint32_t *keys = nullptr, *flags = nullptr, *excl = nullptr, *scan_tmp = nullptr, *owner_counts = nullptr;
+    SortBufs sort;
+  } ev;
   // single-pass training (fr_set_shadow): second copy of Personal_Memory + Adam slots; shadow_dirty = some row's current
   // copy may be the shadow (cleared by shadow_sync, which every reader of the caller's tables runs first)
   float *shP = nullptr, *shM = nullptr, *shV = nullptr; bool shadow_dirty = false;

@@ -81,6 +81,7 @@ void launch_serve_keys(const int32_t* rreq, uint32_t n, uint32_t items_per_rank,
 
 // one warp per requested row; an empty request yields a zero row (staged path).  With peers the row of request slot
 // (source s, j) is stored straight into rank s's receive buffer over NVLink (fused gather + exchange).
+// bf16: 0 fp32 table, 1 bf16 table widened to fp32 rows, 2 bf16 table copied as stored (bf16 rows; staged path only).
 __global__ void __launch_bounds__(FR_THREADS)
 gather_rows_kernel(const float4* __restrict__ R, const int32_t* __restrict__ rreq, uint32_t n, int DV,
                    float4* __restrict__ out, const PeerPtrs peers, uint32_t n_table, int bf16) {
@@ -88,6 +89,12 @@ gather_rows_kernel(const float4* __restrict__ R, const int32_t* __restrict__ rre
   const uint32_t gw = blockIdx.x * FR_WARPS_PER_BLOCK + (threadIdx.x >> 5), nw = gridDim.x * FR_WARPS_PER_BLOCK;
   for (uint32_t r = gw; r < n; r += nw) {
     const int32_t id = rreq[r];
+    if (bf16 == 2) {
+      uint2* d2 = tab_at<true>(out, (size_t)r * DV);
+      for (int i = lane; i < DV; i += 32)
+        d2[i] = (uint32_t)id >= n_table ? make_uint2(0u, 0u) : __ldg(tab_at<true>(R, (size_t)id * DV + i));
+      continue;
+    }
     float4* dst = out + (size_t)r * DV;
     if (peers.world > 0) {
       const uint32_t s = r / (uint32_t)peers.cap, j = r % (uint32_t)peers.cap;

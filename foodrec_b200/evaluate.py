@@ -11,6 +11,8 @@ scoring, dict-dedup and the stable top-K in one launch.  HR / NDCG use the same 
 ``evaluate_full_catalog`` is the full-ranking protocol (extension): the held-out item is ranked
 against EVERY recipe the user did not train on, through the full-catalog top-K with the user's
 training items excluded.
+
+``evaluate_sharded`` is ``evaluate_model`` on row-sharded tables (``sharded.DistRunner`` / ``LocalRunner``).
 """
 from __future__ import annotations
 
@@ -47,6 +49,39 @@ def evaluate_model(sess, model, testRatings, testNegatives, K, dish_to_category)
         raise ValueError("at most 128 candidates per user are supported")
     _, rank = model.engine.eval_sampled_topk(users, cand, ncand, K, cand_cats=ccats)
     rank = rank.cpu().numpy()
+    hits = [1 if r >= 0 else 0 for r in rank]                              # getHitRatio :69-73
+    ndcgs = [math.log(2) / math.log(int(r) + 2) if r >= 0 else 0 for r in rank]   # getNDCG :76-81
+    return hits, ndcgs
+
+
+def evaluate_sharded(runner, testRatings, testNegatives, K, dish_to_category, round_users=None):
+    """``evaluate_model`` on row-sharded tables: ``runner`` is a ``sharded.LocalRunner`` (all ranks in this process) or
+    a ``sharded.DistRunner`` (this process is one rank; every rank passes the same ``testRatings`` / ``testNegatives``).
+    Each test user is evaluated by its owner (user % W) through the runner's ``eval_sampled_topk``; the hits and NDCGs
+    of every user come back in ``testRatings`` order, on every rank, equal to ``evaluate_model`` on the same tables."""
+    import torch
+    users, cand, ncand, ccats = build_candidates(testRatings, testNegatives, dish_to_category)
+    if cand.shape[1] > 128:
+        raise ValueError("at most 128 candidates per user are supported")
+    kw = {} if round_users is None else {"round_users": int(round_users)}
+    local = hasattr(runner, "engs")
+    W = runner.W if local else runner.eng.world
+    owner = users % W
+    per = [np.nonzero(owner == r)[0] for r in range(W)]
+    rank = np.empty(len(users), np.int64)
+    if local:
+        outs = runner.eval_sampled_topk([users[ix] // W for ix in per], [cand[ix] for ix in per], [ncand[ix] for ix in per],
+                                        K, cand_cats=[ccats[ix] for ix in per], **kw)
+        for ix, (_, rk) in zip(per, outs):
+            rank[ix] = rk.cpu().numpy()
+    else:
+        g = runner.eng
+        ix = per[g.rank]
+        _, rk = runner.eval_sampled_topk(users[ix] // W, cand[ix], ncand[ix], K, cand_cats=ccats[ix], **kw)
+        full = torch.zeros(len(users), dtype=torch.int32, device=rk.device)     # gt_rank + 1 at this rank's users
+        full[torch.as_tensor(ix, dtype=torch.int64, device=rk.device)] = rk + 1
+        runner.dist.all_reduce(full)
+        rank[:] = full.cpu().numpy().astype(np.int64) - 1
     hits = [1 if r >= 0 else 0 for r in rank]                              # getHitRatio :69-73
     ndcgs = [math.log(2) / math.log(int(r) + 2) if r >= 0 else 0 for r in rank]   # getNDCG :76-81
     return hits, ndcgs

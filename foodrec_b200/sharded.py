@@ -22,6 +22,11 @@ import torch
 from . import _lib as L
 from .engine import Engine, Hyper, _ptr, exclusion_csr
 
+# test users per round of the sharded sampled evaluation.  A round's received-row buffer (and the served one) holds
+# W * cap rows, cap ~ 1.25 * round_users * stride / W: at 65,536 users x 51 candidates and D = 128, 2.1 GB of fp32 rows
+# each at W = 8, at most 1.7 GB at W = 1 (cap is also bounded by the rows an owner holds)
+EVAL_ROUND_USERS = 65536
+
 
 # ---------------------------------------------------------------------------- host-side layout
 def local_rows(n: int, world: int) -> int:
@@ -71,7 +76,7 @@ class ShardedEngine:
 
     def __init__(self, hyper: Hyper, P_loc, R_loc, Cat, G, rank, world, device="cuda:0", max_rows=1 << 16,
                  cap=None, adam_mode="lazy", item_cats_global=None, user_label_csr_local=None,
-                 max_label_entries=None, adopt=False, single_pass=None, table_dtype="float32"):
+                 max_label_entries=None, adopt=False, single_pass=None, table_dtype="float32", num_users_global=None):
         if not (1 <= world <= 8):
             raise ValueError("1 <= world <= 8")
         self.rank, self.world = rank, world
@@ -81,6 +86,9 @@ class ShardedEngine:
         e = self.e
         self.device = e.device
         self.I_global = None if item_cats_global is None else int(len(item_cats_global))
+        # local rows that hold a user: with the global user count known, the padding rows of the last user shard are
+        # outside Personal_Memory for evaluation (an empty rank list, as for a user past the unsharded table)
+        self.U_valid = e.U if num_users_global is None else min(e.U, len(range(rank, int(num_users_global), world)))
         if item_cats_global is not None:
             # the catalog index of this rank's recipe shard reads the masks of ITS rows (local row k = recipe
             # rank + k*W), never the first rows of the global map: every (re)build of the index uses this slice
@@ -321,6 +329,91 @@ class ShardedEngine:
     def catalog_merge(self, ids, scores):
         return self.e.catalog_merge(ids, scores)
 
+    # sampled evaluation (evaluate.py:35-66) on row-sharded tables ------------------------------------
+    # The user owner plans (its candidates -> one request block per recipe owner + slots into the received rows), the
+    # owners serve the rows, the user owner ranks them with the unsharded engine's kernel (fr_shard_eval_*).
+    def eval_inputs(self, users_local, cand, n_cand, cand_cats=None):
+        """This rank's test users (LOCAL rows), candidates [n, stride] (GLOBAL recipe ids), n_cand [n] and optional
+        category rows [n, stride, 4] on the device.  Host data is range-checked like ``Engine.eval_sampled_topk``
+        does (users against this shard's rows that hold a user, candidates against the global catalog); device tensors
+        are not: there an id outside its table gives an empty rank list (user) or a dropped candidate.  A shard's
+        padding rows hold a user only when the engine was built without ``num_users_global``."""
+        e = self.e
+        if self.I_global is None:
+            raise L.FoodRecError("sharded evaluation needs the global recipe count (item_cats_global)")
+        e._check_ids(users_local, self.U_valid, "test users"); e._check_ids(cand, self.I_global, "candidates")
+        u = e._i32(users_local)
+        cand = torch.as_tensor(np.asarray(cand, np.int32)) if not torch.is_tensor(cand) else cand
+        if cand.dim() != 2 or cand.shape[0] != u.numel():
+            raise ValueError(f"cand must be [n_users, stride]; got {tuple(cand.shape)} for {u.numel()} users")
+        if not 1 <= cand.shape[1] <= 128:
+            raise ValueError("at most 128 candidates per user are supported")
+        n, stride = cand.shape
+        cd = cand.to(self.device, torch.int32).contiguous()
+        nc = e._i32(n_cand)
+        if nc.numel() != n:
+            raise ValueError(f"n_cand has {nc.numel()} entries for {n} users")
+        cc = e._f32(cand_cats, (n, stride, 4))
+        return u, cd, nc, cc
+
+    def eval_cap(self, n_users, stride):
+        """Default per-owner capacity of a round of ``n_users`` users: a rank needs at most n_users*stride distinct
+        recipes and an owner holds at most items_per_rank; random candidates spread over the owners evenly, so 25 %
+        head-room + 256 over the mean covers the imbalance.  Overflow is detected on the device and raised."""
+        ipr = self.e.I
+        return int(max(1, min(ipr, n_users * stride, int(1.25 * n_users * stride / self.world) + 256)))
+
+    def eval_plan(self, cand, n_cand, cap, cand_cats=None, flag=None):
+        """fr_shard_eval_plan of one round: returns the request blocks [W*cap] for the all-to-all.  The slots, the
+        slot -> global id map and the candidates' category rows stay with this engine for eval_rank.  ``flag``
+        (device float [1]) is set to 2 when one owner's block overflows."""
+        e = self.e
+        e.flush()
+        cd = cand.to(self.device, torch.int32).contiguous()
+        n, stride = cd.shape
+        nc = e._i32(n_cand)
+        W, cap = self.world, int(cap)
+        dev = self.device
+        req = torch.empty(W * cap, dtype=torch.int32, device=dev)
+        slot_ids = torch.empty(W * cap, dtype=torch.int32, device=dev)
+        slots = torch.empty((n, stride), dtype=torch.int32, device=dev)
+        cc = e._f32(cand_cats, (n, stride, 4))
+        cats_out = None
+        if cc is None:
+            cc = cats_out = torch.empty((n, stride, 4), dtype=torch.float32, device=dev)
+        if flag is None:
+            flag = torch.zeros(1, dtype=torch.float32, device=dev)
+        L.check(e.handle, e.lib.fr_shard_eval_plan(e.handle, _ptr(cd), _ptr(nc), n, stride, W, self.I_global, cap, _ptr(req),
+                                                   _ptr(slots), _ptr(slot_ids), _ptr(cats_out), _ptr(flag), e._stream()))
+        self._ev = dict(n=n, stride=stride, nc=nc, slots=slots, slot_ids=slot_ids, cats=cc, flag=flag, keep=[cd])
+        return req
+
+    def eval_serve(self, rreq):
+        """fr_shard_eval_serve: the rows the peers requested ([W*cap] local rows, -1 empty), in the table's storage
+        format (fp32, or bf16 as stored), caught up (lazy Adam flushed, single-pass shadow consolidated)."""
+        e = self.e
+        e.flush()
+        rows = torch.empty((rreq.numel(), e.D), dtype=e.R.dtype, device=self.device)
+        L.check(e.handle, e.lib.fr_shard_eval_serve(e.handle, _ptr(rreq), rreq.numel(), _ptr(rows), e._stream()))
+        return rows
+
+    def eval_rank(self, users_local, rbuf, K, ids=None, rank=None, scores=None):
+        """fr_eval_sampled_rows on the rows received for the last eval_plan: ids [n,K] (GLOBAL recipe ids, -1 padded),
+        gt_rank [n], scores [n,stride] (if given) are written into the tensors passed, else allocated."""
+        e = self.e
+        e.flush()
+        ev = self._ev
+        u = e._i32(users_local)
+        n, stride = ev["n"], ev["stride"]
+        assert u.numel() == n
+        ids = torch.empty((n, K), dtype=torch.int32, device=self.device) if ids is None else ids
+        rank = torch.empty(n, dtype=torch.int32, device=self.device) if rank is None else rank
+        L.check(e.handle, e.lib.fr_eval_sampled_rows(e.handle, _ptr(u), self.U_valid, _ptr(ev["slots"]), _ptr(ev["nc"]), n, stride,
+                                                     _ptr(ev["cats"]), _ptr(rbuf), rbuf.shape[0], _ptr(ev["slot_ids"]), K,
+                                                     _ptr(ids), _ptr(rank), _ptr(scores), e._stream()))
+        e._keep = [u, rbuf, ev]
+        return ids, rank
+
 
 # ---------------------------------------------------------------------------- runners
 class DistRunner:
@@ -459,6 +552,38 @@ class DistRunner:
         return g.catalog_merge(rid.view(W, n, K), rsc.view(W, n, K))
 
 
+    def eval_sampled_topk(self, users_local, cand, n_cand, K, cand_cats=None, return_scores=False, round_users=EVAL_ROUND_USERS,
+                          cap=None):
+        """``Engine.eval_sampled_topk`` for this rank's test users (LOCAL rows; candidates GLOBAL recipe ids) on the
+        row-sharded tables: returns ``(ids, gt_rank[, scores])``, bit-identical to the unsharded engine.  Users go in
+        rounds of ``round_users``; every rank walks the same rounds (one all-reduce agrees on their number), and per
+        round runs plan, one all-to-all of request blocks, serve, one all-to-all of rows, rank.  A rank with no test
+        users still serves its peers.  ``cap``: per-owner capacity of a round (default ``eval_cap``); overflow on any
+        rank raises on every rank once all rounds are done."""
+        d, g = self.dist, self.eng
+        u, cd, nc, cc = g.eval_inputs(users_local, cand, n_cand, cand_cats)
+        n, stride = cd.shape
+        dev = getattr(g, "device", u.device)
+        sizes = torch.tensor([n, stride], dtype=torch.int64, device=dev)
+        d.all_reduce(sizes, op=d.ReduceOp.MAX)
+        n_max, stride_max = (int(x) for x in sizes.cpu())
+        rn = max(1, min(int(round_users), n_max))
+        cap = g.eval_cap(rn, stride_max) if cap is None else int(cap)
+        ids, rank, sc = _eval_outputs(n, stride, K, return_scores, dev)
+        flag = torch.zeros(1, dtype=torch.float32, device=dev)
+        for a in range(0, n_max, rn):
+            lo, hi = min(a, n), min(a + rn, n)
+            req = g.eval_plan(cd[lo:hi], nc[lo:hi], cap, None if cc is None else cc[lo:hi], flag)
+            rreq = torch.empty_like(req)
+            d.all_to_all_single(rreq, req)                    # request blocks -> recipe owners
+            rows = g.eval_serve(rreq)
+            rbuf = torch.empty_like(rows)
+            d.all_to_all_single(rbuf, rows)                   # rows -> user owner, block o = owner o's rows
+            g.eval_rank(u[lo:hi], rbuf, K, ids[lo:hi], rank[lo:hi], None if sc is None else sc[lo:hi])
+        d.all_reduce(flag, op=d.ReduceOp.MAX)
+        _eval_check_flag(flag)
+        return (ids, rank, sc) if return_scores else (ids, rank)
+
     def _gather_exclusion(self, exclude, n, dev):
         """This rank's lists for its n query rows -> the CSR of all W*n gathered rows (rank order)."""
         d, W = self.dist, self.eng.world
@@ -474,6 +599,19 @@ class DistRunner:
         d.all_gather_into_tensor(all_ids, pad)
         return concat_csr([all_lens[s * n:(s + 1) * n] for s in range(W)],
                           [all_ids[s * m:s * m + int(per_rank[s])] for s in range(W)])
+
+
+def _eval_outputs(n, stride, K, return_scores, dev):
+    ids = torch.empty((n, K), dtype=torch.int32, device=dev)
+    rank = torch.empty(n, dtype=torch.int32, device=dev)
+    sc = torch.zeros((n, stride), dtype=torch.float32, device=dev) if return_scores else None
+    return ids, rank, sc
+
+
+def _eval_check_flag(flag):
+    if float(flag.max()) != 0:
+        raise L.FoodRecError("sharded evaluation: a rank needed more distinct recipes from one owner than the per-owner "
+                             "capacity of a round; raise cap= or lower round_users=")
 
 
 def concat_csr(lens, ids):
@@ -567,3 +705,28 @@ class LocalRunner:
             sc = torch.stack([lists[w][1][r * n:(r + 1) * n] for w in range(W)])
             out.append(g.catalog_merge(ids, sc))
         return out
+
+    def eval_sampled_topk(self, users_local_per_rank, cand, n_cand, K, cand_cats=None, return_scores=False,
+                          round_users=EVAL_ROUND_USERS, cap=None):
+        """Same protocol as DistRunner.eval_sampled_topk with the all-to-alls as tensor shuffles.  ``cand``, ``n_cand``
+        and ``cand_cats`` (or None) hold one entry per rank.  Returns one ``(ids, gt_rank[, scores])`` per rank."""
+        W = self.W
+        cc_in = cand_cats if cand_cats is not None else [None] * W
+        ins = [g.eval_inputs(u, c, m, x) for g, u, c, m, x in zip(self.engs, users_local_per_rank, cand, n_cand, cc_in)]
+        n_max = max(x[1].shape[0] for x in ins)
+        stride_max = max(x[1].shape[1] for x in ins)
+        rn = max(1, min(int(round_users), n_max))
+        cap = self.engs[0].eval_cap(rn, stride_max) if cap is None else int(cap)
+        outs = [_eval_outputs(x[1].shape[0], x[1].shape[1], K, return_scores, g.device) for g, x in zip(self.engs, ins)]
+        flags = [torch.zeros(1, dtype=torch.float32, device=g.device) for g in self.engs]
+        for a in range(0, n_max, rn):
+            span = [(min(a, x[1].shape[0]), min(a + rn, x[1].shape[0])) for x in ins]
+            reqs = [g.eval_plan(cd[lo:hi], nc[lo:hi], cap, None if cc is None else cc[lo:hi], f)
+                    for g, (u, cd, nc, cc), (lo, hi), f in zip(self.engs, ins, span, flags)]
+            rreqs = [torch.cat([reqs[s].view(W, cap)[r] for s in range(W)]) for r in range(W)]
+            rows = [g.eval_serve(rr) for g, rr in zip(self.engs, rreqs)]
+            rbufs = [torch.cat([rows[o].view(W, cap, -1)[r] for o in range(W)]) for r in range(W)]
+            for g, (u, cd, nc, cc), (lo, hi), rb, (ids, rank, sc) in zip(self.engs, ins, span, rbufs, outs):
+                g.eval_rank(u[lo:hi], rb, K, ids[lo:hi], rank[lo:hi], None if sc is None else sc[lo:hi])
+        _eval_check_flag(torch.cat(flags))
+        return [o if return_scores else o[:2] for o in outs]

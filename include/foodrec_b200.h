@@ -255,6 +255,36 @@ int fr_shard_update(fr_handle h, const fr_batch* b, const fr_shard* sh, int32_t 
 int fr_shard_apply(fr_handle h, const fr_shard* sh, const int32_t* rreq, const float* rgrows, float* out_scalars,
                    fr_stream s);
 
+/* ---- Sampled evaluation (fr_eval_sampled_topk) on row-sharded tables.  A test user is evaluated by its owner
+ * (users = LOCAL rows); its candidates are GLOBAL recipe ids, recipe i lives on rank i % world at local row i / world.
+ *
+ *   fr_shard_eval_plan     this rank's candidates [n_users, cand_stride] -> per owner o the sorted unique requested
+ *                          rows (local rows at o) in req[o*cap .. o*cap+cap) (-1 padded: the training step's request
+ *                          layout), slots [n_users, cand_stride] = the candidate's row in the received buffer
+ *                          (o*cap + k, -1 for j >= n_cand, ids < 0 or >= num_items_global), slot_ids [world*cap] =
+ *                          slot -> global id (-1 unused); cand_cats_out [n_users, cand_stride, 4] (nullable) = the
+ *                          global item_cats rows of the candidates.  More than cap distinct recipes of one owner set
+ *                          *out_flag = 2 (never reset here) and drop the excess candidates.
+ *     all_to_all(req)                                   -> rreq
+ *   fr_shard_eval_serve    owner: rows[n, D] = R[rreq] in the table's storage format (fp32, or bf16 as stored), a
+ *                          zero row for -1.  Lazy Adam: call fr_adam_flush first, as before any read of the tables.
+ *     all_to_all(rows)                                  -> rbuf
+ *   fr_eval_sampled_rows   fr_eval_sampled_topk with cand = slots and the recipe rows taken from rbuf [n_rows, D]
+ *                          (same storage format); cand_cats is required; topk_ids come back as global ids.
+ *                          user_rows (<= Personal_Memory rows) = the local rows that hold a user: a user row at or past
+ *                          it (the padding of the last user shard) gets an empty rank list, as a user past the table
+ *                          does unsharded.
+ *
+ * Ids, gt_rank and scores equal the unsharded engine's bit for bit. */
+int fr_shard_eval_plan(fr_handle h, const int32_t* cand, const int32_t* n_cand, int32_t n_users, int32_t cand_stride,
+                       int32_t world, int32_t num_items_global, int32_t cap, int32_t* req, int32_t* slots,
+                       int32_t* slot_ids, float* cand_cats_out, float* out_flag, fr_stream s);
+int fr_shard_eval_serve(fr_handle h, const int32_t* rreq, int32_t n, void* rows, fr_stream s);
+int fr_eval_sampled_rows(fr_handle h, const int32_t* users, int32_t user_rows, const int32_t* slots,
+                         const int32_t* n_cand, int32_t n_users, int32_t cand_stride, const float* cand_cats, const void* rows, int32_t n_rows,
+                         const int32_t* slot_ids, int32_t K, int32_t* topk_ids, int32_t* gt_rank, float* scores,
+                         fr_stream s);
+
 /* ---- Full-catalog top-K (extension; definition = inference :56-97 over EVERY recipe, the
  * K best by (score desc, id asc)).  The dense contraction runs in bf16 on tcgen05 as a FILTER
  * with a proven error bound; survivors are re-scored in fp64 from the fp32 tables, so ids are
