@@ -7,11 +7,11 @@ Train_recommender.py, and the explicit ``Engine`` underneath.  Importing the pac
 needs neither a GPU nor the built library; using it needs both (no fallback).
 """
 from .data import Dataset, InstanceStream, build_instances
-from .engine import Engine, Hyper
+from .engine import Engine, Hyper, history_csr
 from .evaluate import evaluate_full_catalog, evaluate_model, evaluate_sharded
 from .model import ConfigProto, Model, Saver, Session, global_variables_initializer, latest_checkpoint
 
 __all__ = ["Engine", "Hyper", "Model", "Session", "Saver", "ConfigProto", "evaluate_model", "evaluate_full_catalog",
-           "evaluate_sharded", "Dataset", "InstanceStream",
+           "evaluate_sharded", "Dataset", "InstanceStream", "history_csr",
            "build_instances",
            "global_variables_initializer", "latest_checkpoint"]

@@ -13,6 +13,7 @@ FR_SGD, FR_ADAGRAD, FR_RMSPROP, FR_ADAM = 0, 1, 2, 3
 FR_ADAM_DENSE, FR_ADAM_LAZY_EXACT, FR_ADAM_LAZY_SERIES = 0, 1, 2
 FR_POINTWISE, FR_BPR = 0, 1
 FR_TABLE_F32, FR_TABLE_BF16 = 0, 1
+FR_SAMPLE_NEG, FR_SAMPLE_BPR, FR_SAMPLE_POINTWISE, FR_SAMPLE_CAND = 0, 1, 2, 3
 (FR_OUT_LOSS, FR_OUT_NORM, FR_OUT_SCALE, FR_OUT_GENERAL, FR_OUT_PERSONAL, FR_OUT_LR,
  FR_OUT_UNIQ_USERS, FR_OUT_UNIQ_ITEMS, FR_OUT_LABEL_ENTRIES, FR_OUT_OVERFLOW) = range(10)
 FR_OUT_COUNT = 12
@@ -97,6 +98,9 @@ _PROTOS = {
     "fr_sample_negatives": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_void_p, C.c_void_p]),
     "fr_sample_bpr_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64, C.c_int64,
                                       C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_set_user_history": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "fr_sample_batch": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint64,
+                                  C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "fr_philox4x32_10": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "fr_shard_packed_len": (C.c_int64, [C.c_void_p]),
     "fr_shard_route_block": (C.c_int64, [C.POINTER(fr_batch), C.c_int32]),

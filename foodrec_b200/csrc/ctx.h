@@ -91,6 +91,9 @@ struct fr_ctx {
   bool table_bf16 = false;          // fr_set_table_format: Personal_Memory and Recipe_Embedding are stored in bf16
   bool health_blend = false;        // fr_set_health_blend: inference scores P[u] + alpha * mean G[labels(u)]
   fr::CatalogWs* cat = nullptr;     // full-catalog top-K (catalog.cu): index + pass workspace
+  // fr_set_user_history: caller-owned CSR over Personal_Memory rows the sampler rejects negatives from (sampler.cu)
+  const int32_t *hist_off = nullptr, *hist_ids = nullptr;
+  uint32_t* hist_flag = nullptr;    // its validation flag
   // staging for fr_train_step_host
   void* stage = nullptr; size_t stage_bytes = 0;
   // fr_feed_prefetch: two staging slots filled on a private copy stream while the previous step computes

@@ -79,6 +79,55 @@ def exclusion_csr(exclude, n):
     return off.astype(np.int32), ids.astype(np.int32)
 
 
+def history_csr(history, num_users):
+    """Per-user histories (the recipes each user trained on) as the CSR the sampler reads: ``(offsets int32
+    [num_users+1], ids int32 [nnz])``, every row sorted ascending (duplicates kept).
+
+    ``history`` is the reference's ``trainMatrix`` -- a dict ``{str(user): [recipe ids]}`` (int keys work too; users
+    that are absent have an empty history) -- or a tuple ``(offsets, ids)`` over the ``num_users`` users, in any order
+    within a row.  Raises IndexError for a user outside ``[0, num_users)``, ValueError for malformed offsets, a user
+    given twice, ids that do not fit int32 or more than 2^31 - 1 ids."""
+    num_users = int(num_users)
+    if isinstance(history, dict):
+        rows = {}
+        for k, v in history.items():
+            try:
+                u = int(k)
+            except (TypeError, ValueError):
+                raise ValueError(f"history: user key {k!r} is not an integer") from None
+            if not 0 <= u < num_users:
+                raise IndexError(f"history: user {u} outside [0, {num_users})")
+            if u in rows:
+                raise ValueError(f"history: user {u} is given twice")
+            r = np.asarray(v.cpu().numpy() if torch.is_tensor(v) else v).reshape(-1)
+            rows[u] = r if r.size else r.astype(np.int64)
+        cnt = np.zeros(num_users, np.int64)
+        for u, r in rows.items():
+            cnt[u] = r.size
+        off = np.zeros(num_users + 1, np.int64)
+        off[1:] = np.cumsum(cnt)
+        order = sorted(rows)
+        ids = np.concatenate([rows[u] for u in order]) if order else np.zeros(0, np.int64)
+    elif isinstance(history, tuple) and len(history) == 2:
+        off, ids = ((x.cpu().numpy() if torch.is_tensor(x) else np.asarray(x)).reshape(-1) for x in history)
+    else:
+        raise TypeError("history must be a {user: [recipe ids]} dict or an (offsets, ids) tuple")
+    if off.size and not np.issubdtype(off.dtype, np.integer) or ids.size and not np.issubdtype(ids.dtype, np.integer):
+        raise TypeError("history offsets and ids must be integers")
+    off = off.astype(np.int64); ids = ids.astype(np.int64)
+    if off.shape != (num_users + 1,):
+        raise ValueError(f"history offsets: {off.size} entries for {num_users} users (want {num_users + 1})")
+    if off[0] != 0 or off[-1] != ids.size or (np.diff(off) < 0).any():
+        raise ValueError(f"history offsets must start at 0, be non-decreasing and end at len(ids) = {ids.size}")
+    if ids.size >= 2**31:
+        raise ValueError("history: more than 2^31 - 1 ids")
+    if ids.size and (ids.min() < -2**31 or ids.max() >= 2**31):
+        raise ValueError("history ids must fit int32")
+    row = np.repeat(np.arange(num_users, dtype=np.int64), np.diff(off))
+    ids = ids[np.lexsort((ids, row))]
+    return off.astype(np.int32), ids.astype(np.int32)
+
+
 class Engine:
     def __init__(self, hyper: Hyper, P, R, Cat, G, device="cuda:0", max_rows=1 << 16,
                  max_label_entries=None, adam_mode="lazy", item_cats=None, user_labels=None,
@@ -511,34 +560,89 @@ class Engine:
                          "list_capacity", "fallback_blocks"), list(v)))
 
     # ------------------------------------------------------------------ 1:N negative sampling
-    def sample_negatives(self, pos_items, n_neg, seed, sample_offset=0):
-        """int32 [n, n_neg] device: counter-based (Philox4x32-10) uniform negatives != positive;
-        the same ids oracle/sampler_oracle.sample_negatives draws for (seed, sample index)."""
-        pos = self._i32(pos_items)
-        out = torch.empty((pos.numel(), int(n_neg)), dtype=torch.int32, device=self.device)
-        L.check(self.handle, self.lib.fr_sample_negatives(self.handle, _ptr(pos), pos.numel(), int(n_neg), int(seed) & (2**64 - 1),
-                                                          int(sample_offset), _ptr(out), self._stream()))
-        self._keep = [pos]
-        return out
+    def set_user_history(self, history):
+        """The recipes each user must not get as a sampled negative (normally its training recipes, the reference's
+        ``trainMatrix``): a ``{str(user): [ids]}`` dict or ``(offsets, ids)`` (:func:`history_csr`), one row per
+        Personal_Memory row.  CUDA tensors ``(offsets, ids)`` are used in place (rows must already be ascending: the
+        library checks and raises).  ``None`` clears it.  Synchronises once (the library validates the rows)."""
+        if history is None:
+            L.check(self.handle, self.lib.fr_set_user_history(self.handle, None, None, self._stream()))
+            self._history = None
+            return
+        if (isinstance(history, tuple) and len(history) == 2 and all(torch.is_tensor(x) and x.is_cuda for x in history)):
+            off, ids = history
+            if off.numel() != self.U + 1:
+                raise ValueError(f"history offsets: {off.numel()} entries for {self.U} users (want {self.U + 1})")
+            off, ids = self._i32(off), self._i32(ids)
+        else:
+            off, ids = (torch.as_tensor(x).to(self.device) for x in history_csr(history, self.U))
+        if ids.numel() == 0:
+            ids = torch.zeros(1, dtype=torch.int32, device=self.device)        # never NULL: NULL clears
+        self._history = None
+        L.check(self.handle, self.lib.fr_set_user_history(self.handle, _ptr(off), _ptr(ids), self._stream()))
+        self._history = (off, ids)                   # the library reads them in place
 
-    def sample_bpr_batch(self, users, pos_items, n_neg, seed, sample_offset=0, num_items=0):
+    def _sample(self, layout, users, anchors, n_neg, seed, sample_offset, num_items, exclude_seen):
+        """fr_sample_batch -> (out_users, out_items, out_labels) in ``layout``'s shapes (None where unused)."""
+        pos = self._i32(anchors)
+        u = None if users is None else self._i32(users)
+        if u is not None and u.numel() != pos.numel():
+            raise ValueError(f"{u.numel()} users for {pos.numel()} anchors")
+        n, k = pos.numel(), int(n_neg)
+        dev, i32 = self.device, torch.int32
+        ou = ol = None
+        if layout == L.FR_SAMPLE_NEG:
+            oi = torch.empty((n, k), dtype=i32, device=dev)
+        elif layout == L.FR_SAMPLE_BPR:
+            ou, oi = torch.empty(n * k, dtype=i32, device=dev), torch.empty(2 * n * k, dtype=i32, device=dev)
+        elif layout == L.FR_SAMPLE_POINTWISE:
+            ou, oi = torch.empty(n * (1 + k), dtype=i32, device=dev), torch.empty(n * (1 + k), dtype=i32, device=dev)
+            ol = torch.empty(n * (1 + k), dtype=torch.float32, device=dev)
+        else:
+            oi = torch.empty((n, 1 + k), dtype=i32, device=dev)
+        L.check(self.handle, self.lib.fr_sample_batch(self.handle, int(layout), _ptr(u), _ptr(pos), n, k, int(seed) & (2**64 - 1),
+                                                      int(sample_offset), int(num_items), int(bool(exclude_seen)), _ptr(ou),
+                                                      _ptr(oi), _ptr(ol), self._stream()))
+        self._keep = [u, pos]
+        return ou, oi, ol
+
+    def sample_negatives(self, pos_items, n_neg, seed, sample_offset=0, exclude_seen=False, users=None):
+        """int32 [n, n_neg] device: counter-based (Philox4x32-10) uniform negatives != positive;
+        the same ids oracle/sampler_oracle.sample_negatives draws for (seed, sample index).
+        ``exclude_seen``: also never one of ``users[s]``'s history (set_user_history)."""
+        return self._sample(L.FR_SAMPLE_NEG, users, pos_items, n_neg, seed, sample_offset, 0, exclude_seen)[1]
+
+    def sample_bpr_batch(self, users, pos_items, n_neg, seed, sample_offset=0, num_items=0, exclude_seen=False):
         """(users [n*n_neg], items [2*n*n_neg]) int32 device: the 1:n_neg BPR batch of n positives -- every (user,
         positive) repeated against n_neg sampled negatives (the draws of ``sample_negatives``), laid out as the step
         consumes it.  ``num_items``: catalog size to draw from (0 = this engine's; a row-sharded rank passes the global one)."""
-        u, pos = self._i32(users), self._i32(pos_items)
-        n = pos.numel()
-        ou = torch.empty(n * int(n_neg), dtype=torch.int32, device=self.device)
-        oi = torch.empty(2 * n * int(n_neg), dtype=torch.int32, device=self.device)
-        L.check(self.handle, self.lib.fr_sample_bpr_batch(self.handle, _ptr(u), _ptr(pos), n, int(n_neg), int(seed) & (2**64 - 1),
-                                                          int(sample_offset), int(num_items), _ptr(ou), _ptr(oi), self._stream()))
-        self._keep = [u, pos]
+        ou, oi, _ = self._sample(L.FR_SAMPLE_BPR, users, pos_items, n_neg, seed, sample_offset, num_items, exclude_seen)
         return ou, oi
 
-    def train_step_sampled(self, users, pos_items, n_neg, seed, sample_offset=0, **kw):
-        """One BPR step with n_neg sampled negatives per positive: the batch of B positives becomes
-        B*n_neg triples (u, i+, i-_j) drawn on the device (resident side tables required)."""
-        uu, items = self.sample_bpr_batch(users, pos_items, n_neg, seed, sample_offset)
-        return self._step_dev(L.FR_BPR, uu.numel(), uu, items, None, None, None, None, **kw)
+    def sample_pointwise_batch(self, users, pos_items, n_neg, seed, sample_offset=0, num_items=0, exclude_seen=False):
+        """(users, items, labels) [n*(1+n_neg)] device: the reference's pointwise instances with fresh negatives --
+        per positive the row (u, i+, 1) followed by (u, i-_j, 0) for its n_neg sampled negatives (the draws of
+        ``sample_negatives``), the layout a pointwise step consumes."""
+        return self._sample(L.FR_SAMPLE_POINTWISE, users, pos_items, n_neg, seed, sample_offset, num_items, exclude_seen)
+
+    def sample_eval_candidates(self, users, held_out, n_neg=50, seed=0, sample_offset=0, exclude_seen=True, num_items=0):
+        """The reference's sampled-evaluation lists for test users (``evaluate.py:39-51``: the held-out item and 50
+        negatives the user never trained on), drawn on the device: ``cand`` int32 [n, 1+n_neg] = [held-out,
+        negatives...] and ``n_cand`` int32 [n], ready for ``eval_sampled_topk``."""
+        _, cand, _ = self._sample(L.FR_SAMPLE_CAND, users, held_out, n_neg, seed, sample_offset, num_items, exclude_seen)
+        return cand, torch.full((cand.shape[0],), cand.shape[1], dtype=torch.int32, device=self.device)
+
+    def train_step_sampled(self, users, pos_items, n_neg, seed, sample_offset=0, mode="bpr", exclude_seen=False, **kw):
+        """One step with n_neg sampled negatives per positive, drawn on the device (resident side tables required).
+        ``mode="bpr"``: B positives -> B*n_neg triples (u, i+, i-_j); ``mode="pointwise"``: B*(1+n_neg) labelled rows
+        (``sample_pointwise_batch``), the reference's objective.  ``exclude_seen``: negatives skip the user's history."""
+        if mode == "bpr":
+            uu, items = self.sample_bpr_batch(users, pos_items, n_neg, seed, sample_offset, exclude_seen=exclude_seen)
+            return self._step_dev(L.FR_BPR, uu.numel(), uu, items, None, None, None, None, **kw)
+        if mode == "pointwise":
+            uu, items, labels = self.sample_pointwise_batch(users, pos_items, n_neg, seed, sample_offset, exclude_seen=exclude_seen)
+            return self._step_dev(L.FR_POINTWISE, uu.numel(), uu, items, None, labels, None, None, **kw)
+        raise ValueError("mode must be 'bpr' or 'pointwise'")
 
     def philox(self, ctr_key):
         ck = torch.as_tensor(np.ascontiguousarray(np.asarray(ctr_key, np.uint32)).view(np.int32)).to(self.device)

@@ -20,7 +20,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .engine import Engine, Hyper, _ptr, exclusion_csr
+from .engine import Engine, Hyper, _ptr, exclusion_csr, history_csr
 
 # test users per round of the sharded sampled evaluation.  A round's received-row buffer (and the served one) holds
 # W * cap rows, cap ~ 1.25 * round_users * stride / W: at 65,536 users x 51 candidates and D = 128, 2.1 GB of fp32 rows
@@ -89,6 +89,7 @@ class ShardedEngine:
         # local rows that hold a user: with the global user count known, the padding rows of the last user shard are
         # outside Personal_Memory for evaluation (an empty rank list, as for a user past the unsharded table)
         self.U_valid = e.U if num_users_global is None else min(e.U, len(range(rank, int(num_users_global), world)))
+        self.U_global = None if num_users_global is None else int(num_users_global)
         if item_cats_global is not None:
             # the catalog index of this rank's recipe shard reads the masks of ITS rows (local row k = recipe
             # rank + k*W), never the first rows of the global map: every (re)build of the index uses this slice
@@ -154,16 +155,47 @@ class ShardedEngine:
         self._pending = (L.fr_batch(mode, B, _ptr(users_local), _ptr(items), _ptr(None), _ptr(labels), _ptr(None), _ptr(None)),
                          self._shard(global_batch if global_batch is not None else B), [users_local, items, labels])
 
-    def set_batch_sampled(self, users_local, pos_items_global, n_neg, seed, sample_offset=0, global_batch=None, num_items=None):
-        """1:n_neg BPR batch drawn on the device (fr_sample_bpr_batch): n (user, positive) pairs of THIS rank's users ->
-        n*n_neg triples, negatives uniform over the GLOBAL catalog.  ``sample_offset`` = the global index of this
-        rank's first pair, so the draws do not depend on how the pairs are spread over the ranks."""
+    def set_batch_sampled(self, users_local, pos_items_global, n_neg, seed, sample_offset=0, global_batch=None, num_items=None,
+                          mode="bpr", exclude_seen=False):
+        """1:n_neg batch drawn on the device (fr_sample_batch): n (user, positive) pairs of THIS rank's users ->
+        n*n_neg BPR triples (``mode="bpr"``) or n*(1+n_neg) labelled pointwise rows (``mode="pointwise"``), negatives
+        uniform over the GLOBAL catalog (``exclude_seen``: outside the user's history, ``set_user_history``).
+        ``sample_offset`` = the global index of this rank's first pair, so the draws do not depend on how the pairs are
+        spread over the ranks.  ``global_batch``: triples / rows summed over the ranks."""
         ni = num_items if num_items is not None else self.I_global
         if ni is None:
             raise ValueError("set_batch_sampled needs the global recipe count (num_items= or item_cats_global)")
-        uu, items = self.e.sample_bpr_batch(users_local, pos_items_global, n_neg, seed, sample_offset, num_items=ni)
+        if mode == "bpr":
+            uu, items = self.e.sample_bpr_batch(users_local, pos_items_global, n_neg, seed, sample_offset, num_items=ni,
+                                                exclude_seen=exclude_seen)
+            labels, fr_mode = None, L.FR_BPR
+        elif mode == "pointwise":
+            uu, items, labels = self.e.sample_pointwise_batch(users_local, pos_items_global, n_neg, seed, sample_offset,
+                                                              num_items=ni, exclude_seen=exclude_seen)
+            fr_mode = L.FR_POINTWISE
+        else:
+            raise ValueError("mode must be 'bpr' or 'pointwise'")
         B = uu.numel()
-        self.set_batch_dev(L.FR_BPR, B, uu, items, global_batch=global_batch if global_batch is not None else B)
+        self.set_batch_dev(fr_mode, B, uu, items, labels, global_batch=global_batch if global_batch is not None else B)
+
+    def set_user_history(self, global_history):
+        """The history of every user (GLOBAL user ids, GLOBAL recipe ids: the reference's ``trainMatrix`` or an
+        ``(offsets, ids)`` CSR over all users, :func:`history_csr`); this rank keeps its own users' rows."""
+        if global_history is None:
+            self.e.set_user_history(None)
+            return
+        n_users = self.U_global if self.U_global is not None else self.e.U * self.world
+        off, ids = history_csr(global_history, n_users)
+        self.e.set_user_history(shard_label_csr(off, ids, self.rank, self.world, n_users))
+
+    def sample_eval_candidates(self, users_local, held_out_global, n_neg=50, seed=0, sample_offset=0, exclude_seen=True):
+        """``Engine.sample_eval_candidates`` for this rank's test users (LOCAL rows) over the GLOBAL catalog: ``(cand,
+        n_cand)`` for ``eval_sampled_topk``.  With ``sample_offset`` = the global index of this rank's first test user,
+        the ranks' lists are, together, the lists one engine draws."""
+        if self.I_global is None:
+            raise ValueError("sample_eval_candidates needs the global recipe count (item_cats_global)")
+        return self.e.sample_eval_candidates(users_local, held_out_global, n_neg, seed, sample_offset, exclude_seen,
+                                             num_items=self.I_global)
 
     def set_batch_raw(self, batch, keep, global_batch):
         """An fr_batch built by the caller (device pointers) -- e.g. the reference's dense feed."""

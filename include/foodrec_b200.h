@@ -362,6 +362,32 @@ int fr_sample_negatives(fr_handle h, const int32_t* pos_items, int64_t n, int32_
 int fr_sample_bpr_batch(fr_handle h, const int32_t* users, const int32_t* pos_items, int64_t n, int32_t n_neg,
                         uint64_t seed, uint64_t sample_offset, int64_t num_items, int32_t* out_users,
                         int32_t* out_items, fr_stream s);
+/* Negatives that skip each user's history (e.g. the training recipes, the reference's trainMatrix): its listed
+ * negatives are unseen items (Train_recommender.py:86-93, evaluate.py:39-51), a uniform draw is not.
+ * fr_set_user_history: the history as a CSR over this handle's Personal_Memory rows (local rows on a row-sharded rank):
+ * off [num_users+1], ids [off[num_users]] int32, device, caller-owned (kept, not copied: leave it in place while it is
+ * set), ids in the space the negatives are drawn from (GLOBAL recipe ids on a row-sharded rank).  Checked by one kernel
+ * (off[0] == 0, non-decreasing offsets, every row ascending; duplicates allowed) whose flag is read back, so the call
+ * synchronises the stream once; a violation returns FR_ERR_ARG and leaves the handle without a history.  NULL, NULL
+ * clears it.
+ * fr_sample_batch: for sample s (index g = sample_offset + s), user u = users[s], anchor p = anchors[s] in [0, I) and
+ * negative j, with H(u) = the history when use_history (a user outside Personal_Memory has an empty one) else empty:
+ *   1. the first of 16 attempts cand = mulhi32(philox((g_lo, g_hi, j, a), seed).x0, I) with cand != p, cand not in H(u);
+ *   2. else the first c of (p+1) % I, (p+2) % I, ... with c != p, c not in H(u);
+ *   3. else (H(u) and p cover the catalog) (p+1) % I.
+ * With an empty history this is fr_sample_negatives' rule, bit for bit.  Negatives of one sample may repeat.
+ * num_items as fr_sample_bpr_batch.  use_history without a history set is FR_ERR_STATE.  Layouts:
+ *   FR_SAMPLE_NEG        out_items [n, n_neg] (= fr_sample_negatives; users only read with use_history)
+ *   FR_SAMPLE_BPR        = fr_sample_bpr_batch (out_users [n*n_neg], out_items [2*n*n_neg], 8-byte aligned)
+ *   FR_SAMPLE_POINTWISE  n*(1+n_neg) rows: row s*(1+n_neg) = (users[s], p, 1.0), then (users[s], negative_j, 0.0):
+ *                        out_users, out_items, out_labels -- a pointwise fr_batch with write_sign NULL
+ *   FR_SAMPLE_CAND       out_items [n, 1+n_neg] = [p, negatives...]: candidates for fr_eval_sampled_topk /
+ *                        fr_shard_eval_plan (p = the held-out item) */
+enum { FR_SAMPLE_NEG = 0, FR_SAMPLE_BPR = 1, FR_SAMPLE_POINTWISE = 2, FR_SAMPLE_CAND = 3 };
+int fr_set_user_history(fr_handle h, const int32_t* off, const int32_t* ids, fr_stream s);
+int fr_sample_batch(fr_handle h, int32_t layout, const int32_t* users, const int32_t* anchors, int64_t n, int32_t n_neg,
+                    uint64_t seed, uint64_t sample_offset, int64_t num_items, int32_t use_history, int32_t* out_users,
+                    int32_t* out_items, float* out_labels, fr_stream s);
 /* The raw generator (known-answer tests): ctr_key [n,6] = counter[4], key[2] -> out [n,4]. */
 int fr_philox4x32_10(fr_handle h, const uint32_t* ctr_key, int32_t n, uint32_t* out, fr_stream s);
 
