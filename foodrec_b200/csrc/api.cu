@@ -330,6 +330,154 @@ extern "C" int fr_adam_flush(fr_handle h, fr_stream s) {
   return FR_OK;
 }
 
+// ---------------------------------------------------------------- phases of a training step
+// Built once for both callers: fr_train_step reads the tables, fr_shard_forward / fr_shard_update the rows this rank
+// planned and received (StepRows).  Launch errors are left for the caller's FR_CHECK_LAUNCH.
+
+// The single-pass step: forward + Personal_Memory update in one kernel on the double-buffered table (train_seg.cu)
+bool single_pass(const fr_ctx* h) {
+  return h->cfg.learner == FR_ADAM && h->cfg.adam_mode != FR_ADAM_DENSE && h->shP && !getenv("FOODREC_TWO_PASS");
+}
+
+// Storage of the tables a pass reads: 0 fp32 P and R, 1 bf16 P and R, 2 bf16 P + fp32 R (received rows).  The passes
+// that read only recipe rows (LabelPolParams, ItemPolParams) read bf16 ones for code 1 alone.
+int tab_code(const fr_ctx* h, bool R_is_table) { return !h->table_bf16 ? 0 : R_is_table ? 1 : 2; }
+
+// Entry list of the General_Memory pass: non-zeros of the label feed -> (label, row, coef), sorted by label
+int label_entries(fr_ctx* h, const StepRows& r, const Launch& l) {
+  LabelEmitParams ep{};
+  ep.S = r.S; ep.group = r.group; ep.L = h->mc.L; ep.users = r.users;
+  ep.user_labels = r.user_labels; ep.lab_off = h->tab.user_label_off; ep.lab_idx = h->tab.user_label_idx;
+  ep.ws_row = r.ws_row; ep.counts = h->counts; ep.offs = h->offs;
+  ep.ent_key = h->ent_key; ep.ent_row = h->ent_row; ep.ent_coef = h->ent_coef;
+  ep.cap = (uint32_t)h->sortL.cap; ep.n_entries = h->n_entries; ep.out = r.out;
+  launch_label_count(ep, l);
+  exclusive_scan_u32(h->counts, h->offs, (uint32_t)r.S, h->scan_tmp, h->n_entries, l.st);
+  launch_label_emit(ep, l);
+  return radix_sort_pairs(h->sortL, h->ent_key, ep.cap, h->n_entries, bits_for(h->mc.L), l.st, h->sm_count);
+}
+
+// General_Memory: segment reduce of the label entries (sort result rl) by label into r.G.  It reads pre-step state only.
+// (Round 2 tried a shared-memory scatter with one owner warp per label instead -- no sort, no entry list: measured
+// 354 us + 25 us against this pass's 254 us at 524k rows; see DESIGN.md "measured and rejected".)
+void label_pass(fr_ctx* h, const StepRows& r, int rl, const Launch& l) {
+  SegCommon c{};
+  c.keys = h->sortL.k[rl]; c.perm = h->sortL.v[rl]; c.n_dev = h->n_entries; c.n_host = (uint32_t)h->sortL.cap;
+  c.pieces = h->pieces_g; c.uniq_counter = nullptr;
+  c.long_list = h->long_list; c.long_count = h->counters + 2; c.long_cap = h->long_cap;
+  LabelPolParams lp{};
+  lp.G = r.G; lp.R = r.R; lp.cat = h->cat_pre;
+  lp.ent_row = h->ent_row; lp.ent_coef = h->ent_coef; lp.items = r.items; lp.cats = r.cats;
+  lp.cats_by_item = r.cats_by_item; lp.mc = h->mc; lp.tab = tab_code(h, r.R_is_table) == 1;
+  launch_label_pass(h->NV, c, lp, l);
+}
+
+static SegCommon user_seg(fr_ctx* h, const StepRows& r) {   // the rows by user
+  SegCommon c{};
+  c.keys = r.ukeys; c.perm = r.uperm; c.n_dev = nullptr; c.n_host = (uint32_t)r.S;
+  c.uniq_counter = h->counters + 0; c.pieces = h->pieces_u;
+  return c;
+}
+
+// Forward, loss, per-slice norms, dCat partials, z stash.  Single-pass (fused): also the segment reduce by user and Adam
+// with the clip scale speculated = 1, new rows into the other copy of the double-buffered Personal_Memory; user_update
+// commits them once the norm is known.  l.mid: recorded between the single-pass kernel and its crossing-run combine.
+// Returns the grid, whose per-block partials finalize reduces.
+int forward(fr_ctx* h, const StepRows& r, bool fused, const OptConsts& oc, const Launch& l) {
+  const fr_tables& T = h->tab;
+  if (fused) {
+    FusedParams fz{};
+    fz.P[0] = (float4*)T.P; fz.m[0] = (float4*)T.s1_P; fz.v[0] = (float4*)T.s2_P;
+    fz.P[1] = (float4*)h->shP; fz.m[1] = (float4*)h->shM; fz.v[1] = (float4*)h->shV;
+    fz.last = T.last_P; fz.R = r.R; fz.cat = h->cat_pre;
+    fz.items = r.items; fz.cats = r.cats; fz.cats_by_item = r.cats_by_item; fz.labels = r.labels;
+    fz.a = h->mc.a; fz.oma = h->mc.oma; fz.Bnorm = r.Bnorm;
+    fz.g = h->g; fz.z = h->z; fz.scores = r.scores;
+    fz.part_loss = h->part_loss; fz.part_nrm = h->part_nrm; fz.part_gcat = h->part_gcat;
+    fz.mc = h->mc; fz.oc = oc;
+    const int grid = user_fused_grid((uint32_t)r.S, h->sm_count);
+    launch_user_fused(h->NV, r.group, user_seg(h, r), fz, grid, l);
+    h->shadow_dirty = true;
+    return grid;
+  }
+  FwdParams fp{};
+  fp.P = (const float4*)T.P; fp.R = r.R; fp.cat = h->cat_pre; fp.DV = h->mc.DV; fp.B = r.B; fp.Bnorm = r.Bnorm;
+  fp.users = r.users; fp.items = r.items; fp.cats = r.cats; fp.cats_by_item = r.cats_by_item;
+  fp.labels = r.labels; fp.a = h->mc.a; fp.oma = h->mc.oma;
+  fp.g = h->g; fp.z = h->z; fp.scores = r.scores;
+  fp.part_loss = h->part_loss; fp.part_nrm = h->part_nrm; fp.part_gcat = h->part_gcat;
+  fp.lazy = h->cfg.learner == FR_ADAM && h->cfg.adam_mode != FR_ADAM_DENSE;
+  fp.mP = (const float4*)T.s1_P; fp.vP = (const float4*)T.s2_P; fp.lastP = T.last_P; fp.oc = oc;
+  fp.tab = tab_code(h, r.R_is_table);
+  const int grid = fwd_train_grid(r.B, h->sm_count);
+  launch_fwd_train(h->NV, r.group, fp, grid, l);
+  return grid;
+}
+
+// Personal_Memory: segment reduce by user + optimizer, then on personal steps Write_Memory (Model_Recommender.py:149-198)
+// on the optimizer's output, which reads pre-step R, Cat, G.  l.mid: recorded between the user pass's chunk kernel and
+// its combine; before_personal (nullable): recorded after the user pass.
+int user_update(fr_ctx* h, const StepRows& r, bool fused, bool write_personal, const OptConsts& oc, int64_t step,
+                Launch l, cudaEvent_t before_personal) {
+  const fr_tables& T = h->tab;
+  SegCommon c = user_seg(h, r);
+  UserPolParams up{};
+  up.P = (float4*)T.P; up.s1 = (float4*)T.s1_P; up.s2 = (float4*)T.s2_P; up.last = T.last_P;
+  up.R = r.R; up.G = (const float4*)T.G; up.cat = h->cat_pre;
+  up.items = r.items; up.g = h->g; up.cats = r.cats; up.cats_by_item = r.cats_by_item;
+  up.ws_row = r.ws_row; up.out = r.out; up.group = r.group; up.mc = h->mc; up.oc = oc;
+  up.user_labels = r.user_labels; up.lab_off = T.user_label_off; up.lab_idx = T.user_label_idx; up.users = r.users;
+  up.tab = tab_code(h, r.R_is_table);
+  if (r.S == 0) {
+    if (l.mid) cudaEventRecord(l.mid, l.st);
+  } else {
+    if (fused) {
+      // the norm is known.  scale == 1 exactly: the speculative rows become current (stamp bits flipped).  Otherwise
+      // nothing was committed: every row goes back to the caller's tables and the ordinary update pass runs with the
+      // true scale on the g / z the single-pass kernel left (both launches exit at once in the common case).
+      launch_user_commit(c.keys, (uint32_t)r.S, T.last_P, r.out, (int)step, l);
+      launch_shadow_consolidate(T.last_P, h->cfg.num_users, 5 * h->mc.DV, (float4*)T.P, (float4*)T.s1_P,
+                                (float4*)T.s2_P, (const float4*)h->shP, (const float4*)h->shM, (const float4*)h->shV,
+                                r.out, l);
+      c.uniq_counter = nullptr;          // (counted by the single-pass kernel)
+      c.only_if_scaled = r.out;
+    }
+    launch_user_pass(h->NV, c, up, l);
+  }
+  l.mid = nullptr;
+  if (before_personal) cudaEventRecord(before_personal, l.st);
+  if (!write_personal || r.S == 0) return FR_OK;
+  if (fused) { int rc = shadow_sync(h, l.st); if (rc) return rc; }     // the personal pass works on the caller's table
+  c.only_if_scaled = nullptr;                                         // (it always runs, whatever the clip did)
+  const size_t need = (size_t)r.S / 32 + 2;
+  if (need > h->pieces_personal_chunks) {
+    if (h->pieces_personal) { FR_CUDA(h, cudaStreamSynchronize(l.st)); cudaFree(h->pieces_personal); h->pieces_personal = nullptr; }
+    FR_CUDA(h, cudaMalloc(&h->pieces_personal, need * 2 * 10 * h->mc.DV * sizeof(float4)));
+    h->pieces_personal_chunks = need;
+  }
+  c.pieces = h->pieces_personal; c.uniq_counter = nullptr;
+  launch_personal_pass(h->NV, c, up, l);
+  return FR_OK;
+}
+
+// LAZY_SERIES table: every catch-up of this step (target t-1) is done; add the s = t term so that the table serves
+// target t (a personal step's sweep, fr_adam_flush, step t+1).  TF-1.x dense Adam: every untouched row decays this step too.
+void optimizer_tail(fr_ctx* h, const OptConsts& oc, int64_t step, const Launch& l) {
+  const fr_tables& T = h->tab;
+  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_LAZY_SERIES)
+    launch_series_update(h->cser, h->lr_hist, (int)step, h->cfg.adam_beta1, h->cfg.adam_beta2, l);
+  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_DENSE) {
+    launch_adam_sweep((float4*)T.P, (float4*)T.s1_P, (float4*)T.s2_P, T.last_P, h->cfg.num_users, 5 * h->mc.DV, oc, (int)step, l);
+    launch_adam_sweep((float4*)T.R, (float4*)T.s1_R, (float4*)T.s2_R, T.last_R, h->cfg.num_items, h->mc.DV, oc, (int)step, l);
+  }
+}
+
+void step_advance(fr_ctx* h, int64_t step) {
+  h->step = step;
+  h->b1p *= h->cfg.adam_beta1;     // adam.py _finish
+  h->b2p *= h->cfg.adam_beta2;
+}
+
 extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_personal, float* out_scalars,
                              float* out_scores, fr_stream s) {
   if (!h || !h->has_tables) return fail(h, FR_ERR_STATE, "fr_set_tables first");
@@ -357,17 +505,16 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   int rc = ensure_lr_hist(h, step + 1, st); if (rc) return rc;
   const OptConsts oc = make_oc(h, step);
   float* out = out_scalars ? out_scalars : h->out_internal;
-  const float4* cats = (const float4*)(b->cats ? b->cats : T.item_cats);
-  const int cats_by_item = b->cats ? 0 : 1;
+  StepRows r{};
+  r.B = B; r.S = S; r.group = group;
+  r.users = h->users_s; r.items = h->items_s; r.ws_row = h->ws_row;     // range-checked: every kernel below reads these
+  r.R = (const float4*)T.R; r.R_is_table = true;
+  r.cats = (const float4*)(b->cats ? b->cats : T.item_cats); r.cats_by_item = b->cats ? 0 : 1;
+  r.labels = b->labels; r.user_labels = b->user_labels; r.Bnorm = (float)B;
+  r.out = out; r.scores = out_scores ? out_scores : h->scores; r.G = (float4*)T.G;
 
-  fr_ctx::TimingSet* ts = nullptr;
-  if (h->timing) {
-    ts = &h->tsets[h->ts_next++ % h->tsets.size()];
-    timing_collect(h, *ts);
-    ts->used = true;
-  }
-#define FR_MARK(i) do { if (ts) cudaEventRecord(ts->ev[i], st); } while (0)
-  FR_MARK(FR_T_SORT);
+  const StepTiming tm(h, st);
+  tm.mark(FR_T_SORT);
   // 0. pre-step snapshot of Category_Embedding (every read of Cat in this step sees it)
   FR_CUDA(h, cudaMemcpyAsync(h->cat_pre, T.Cat, (size_t)4 * h->mc.D * sizeof(float), cudaMemcpyDeviceToDevice, st));
   FR_CUDA(h, cudaMemsetAsync(h->counters, 0, 4 * sizeof(uint32_t), st));
@@ -376,40 +523,26 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   // 1. row keys, write sign; sort item rows by user and by recipe
   launch_prep_rows(b->mode, B, b->users, b->items, b->labels, b->write_sign, h->cfg.num_users, h->cfg.num_items, h->ukeys,
                    h->ws_row, h->users_s, h->items_s, out + FR_OUT_OVERFLOW, l);
-  const int32_t *users = h->users_s, *items = h->items_s;      // range-checked: every kernel below reads these
-  // 1b. FORK: the General_Memory pass's entry list -- non-zeros of the label feed -> (label, row, coef), sorted by label
-  //     -- depends only on the batch.  It is ~0.1 ms of small latency-bound kernels (count, scan, emit, one radix pass)
-  //     that used to sit on the step's critical path; they now run on a side stream beside the sorts / catch-up /
-  //     forward (which are small or bandwidth-bound) and are joined before the label segment-reduce needs them.
-  int rl = 0;
-  const uint32_t ecap = (uint32_t)h->sortL.cap;
-  {
-    if ((rc = aux_ensure(h))) return rc;
-    FR_CUDA(h, cudaEventRecord(h->aux_fork, st));
-    FR_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->aux_fork, 0));
-    Launch la{h->sm_count, h->aux_stream, nullptr};
-    LabelEmitParams ep{};
-    ep.S = S; ep.group = group; ep.L = h->mc.L; ep.users = users;
-    ep.user_labels = b->user_labels; ep.lab_off = T.user_label_off; ep.lab_idx = T.user_label_idx;
-    ep.ws_row = h->ws_row; ep.counts = h->counts; ep.offs = h->offs;
-    ep.ent_key = h->ent_key; ep.ent_row = h->ent_row; ep.ent_coef = h->ent_coef;
-    ep.cap = ecap; ep.n_entries = h->n_entries; ep.out = out;
-    launch_label_count(ep, la);
-    exclusive_scan_u32(h->counts, h->offs, (uint32_t)S, h->scan_tmp, h->n_entries, h->aux_stream);
-    launch_label_emit(ep, la);
-    rl = radix_sort_pairs(h->sortL, h->ent_key, ecap, h->n_entries, bits_for(h->mc.L), h->aux_stream, h->sm_count);
-    FR_CHECK_LAUNCH(h);
-  }
-  SortJob sj[2] = {{&h->sortU, h->ukeys, (uint32_t)S, nullptr, bits_for(h->cfg.num_users), 0},
-                   {&h->sortI, (const uint32_t*)items, (uint32_t)S, nullptr, bits_for(h->cfg.num_items), 0}};
-  radix_sort_jobs(sj, 2, st, h->sm_count);      // by user and by recipe, sharing their launches
-  const int ru = sj[0].result, ri = sj[1].result;
+  // 1b. FORK: the General_Memory pass's entry list depends only on the batch.  It is ~0.1 ms of small latency-bound
+  //     kernels (count, scan, emit, one radix pass) that used to sit on the step's critical path; they now run on a side
+  //     stream beside the sorts / catch-up / forward (which are small or bandwidth-bound) and are joined before the label
+  //     segment-reduce needs them.
+  if ((rc = aux_ensure(h))) return rc;
+  FR_CUDA(h, cudaEventRecord(h->aux_fork, st));
+  FR_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->aux_fork, 0));
+  const Launch la{h->sm_count, h->aux_stream, nullptr};
+  const int rl = label_entries(h, r, la);
   FR_CHECK_LAUNCH(h);
-  const bool lazy = h->cfg.learner == FR_ADAM && h->cfg.adam_mode != FR_ADAM_DENSE;
-  // single-pass step: forward + Personal_Memory update in one kernel on the double-buffered table (train_seg.cu).
+  SortJob sj[2] = {{&h->sortU, h->ukeys, (uint32_t)S, nullptr, bits_for(h->cfg.num_users), 0},
+                   {&h->sortI, (const uint32_t*)h->items_s, (uint32_t)S, nullptr, bits_for(h->cfg.num_items), 0}};
+  radix_sort_jobs(sj, 2, st, h->sm_count);      // by user and by recipe, sharing their launches
+  const int ri = sj[1].result;
+  r.ukeys = h->sortU.k[sj[0].result]; r.uperm = h->sortU.v[sj[0].result];
+  FR_CHECK_LAUNCH(h);
   // Personal-write steps (16 per run of the reference, Train_recommender.py:169-187) take the two-pass path.
-  const bool fused = lazy && h->shP && !write_personal && !getenv("FOODREC_TWO_PASS");
+  const bool fused = single_pass(h) && !write_personal;
   if (!fused) { rc = shadow_sync(h, st); if (rc) return rc; }
+  const bool lazy = h->cfg.learner == FR_ADAM && h->cfg.adam_mode != FR_ADAM_DENSE;
   if (lazy) {   // recipe rows of this batch must be current before anything reads them
     launch_item_catchup(NV, h->sortI.k[ri], (uint32_t)S, (float4*)T.R, (float4*)T.s1_R, (float4*)T.s2_R,
                         T.last_R, DV, oc, l);
@@ -421,73 +554,29 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   //     on the side stream too, beside the forward / user pass (bandwidth-bound; this pass is issue-bound), and is joined
   //     before the recipe pass overwrites R.
   //     (With fr_timing_enable the pass runs in sequence, so that every phase time is that of its kernels alone.)
-  const bool label_aside = !write_personal && !h->timing && !getenv("FOODREC_LABEL_SERIAL");
-  auto label_pass = [&](Launch& ll) -> int {
-    SegCommon c{};
-    c.keys = h->sortL.k[rl]; c.perm = h->sortL.v[rl]; c.n_dev = h->n_entries; c.n_host = ecap;
-    c.pieces = h->pieces_g; c.uniq_counter = nullptr;
-    c.long_list = h->long_list; c.long_count = h->counters + 2; c.long_cap = h->long_cap;
-    LabelPolParams lp{};
-    lp.G = (float4*)T.G; lp.R = (const float4*)T.R; lp.cat = h->cat_pre;
-    lp.ent_row = h->ent_row; lp.ent_coef = h->ent_coef; lp.items = items; lp.cats = cats;
-    lp.cats_by_item = cats_by_item; lp.mc = h->mc; lp.tab = h->table_bf16 ? 1 : 0;
-    launch_label_pass(NV, c, lp, ll);
-    FR_CHECK_LAUNCH(h);
-    return FR_OK;
-  };
+  const bool label_aside = !write_personal && !h->timing;
   if (label_aside) {
     FR_CUDA(h, cudaEventRecord(h->aux_fork2, st));
     FR_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->aux_fork2, 0));
-    Launch la{h->sm_count, h->aux_stream, nullptr};
-    rc = label_pass(la); if (rc) return rc;
+    label_pass(h, r, rl, la);
     // the `general` fetch = mean(G) (:219) only needs the pass above: off the main stream too
     launch_mean((const float4*)T.G, (int64_t)h->mc.L * 5 * DV, h->mean_partials, out + FR_OUT_GENERAL,
                 (double)h->mc.L * 5.0 * h->mc.D, la);
+    FR_CHECK_LAUNCH(h);
   }
   FR_CUDA(h, cudaEventRecord(h->aux_join, h->aux_stream));
 
-  FR_MARK(FR_T_FWD);
-  int fgrid;
-  SegCommon cu{};
-  cu.keys = h->sortU.k[ru]; cu.perm = h->sortU.v[ru]; cu.n_dev = nullptr; cu.n_host = (uint32_t)S;
-  cu.uniq_counter = h->counters + 0; cu.pieces = h->pieces_u;
-  const bool fin_aside = fused && !h->timing && !getenv("FOODREC_FINALIZE_SERIAL");
-  if (fused) {
-    // 2'. forward + loss + norms + dCat partials + z stash + segment reduce + Adam (clip scale speculated = 1), new rows
-    //     into the other copy of the double-buffered Personal_Memory
-    FusedParams fz{};
-    fz.P[0] = (float4*)T.P; fz.m[0] = (float4*)T.s1_P; fz.v[0] = (float4*)T.s2_P;
-    fz.P[1] = (float4*)h->shP; fz.m[1] = (float4*)h->shM; fz.v[1] = (float4*)h->shV;
-    fz.last = T.last_P; fz.R = (const float4*)T.R; fz.cat = h->cat_pre;
-    fz.items = items; fz.cats = cats; fz.cats_by_item = cats_by_item; fz.labels = b->labels;
-    fz.a = h->mc.a; fz.oma = h->mc.oma; fz.Bnorm = (float)B;
-    fz.g = h->g; fz.z = h->z; fz.scores = out_scores ? out_scores : h->scores;
-    fz.part_loss = h->part_loss; fz.part_nrm = h->part_nrm; fz.part_gcat = h->part_gcat;
-    fz.mc = h->mc; fz.oc = oc;
-    fgrid = user_fused_grid((uint32_t)S, h->sm_count);
-    // (the norm / loss / dCat partials are complete when the kernel ends; its crossing-run combine does not touch them:
-    //  finalize runs beside the combine on a second side stream -- the event is recorded between the two launches)
-    if (fin_aside) l.mid = h->aux2_fork;
-    launch_user_fused(NV, group, cu, fz, fgrid, l);
-    l.mid = nullptr;
-    FR_CHECK_LAUNCH(h);
-    h->shadow_dirty = true;
-  } else {
-  // 2. forward, loss, per-slice norms, dCat partials, z stash
-  FwdParams fp{};
-  fp.P = (const float4*)T.P; fp.R = (const float4*)T.R; fp.cat = h->cat_pre; fp.DV = DV; fp.B = B; fp.Bnorm = (float)B;
-  fp.users = users; fp.items = items; fp.cats = cats; fp.cats_by_item = cats_by_item;
-  fp.labels = b->labels; fp.a = h->mc.a; fp.oma = h->mc.oma;
-  fp.g = h->g; fp.z = h->z; fp.scores = out_scores ? out_scores : h->scores;
-  fp.part_loss = h->part_loss; fp.part_nrm = h->part_nrm; fp.part_gcat = h->part_gcat;
-  fp.lazy = lazy ? 1 : 0; fp.mP = (const float4*)T.s1_P; fp.vP = (const float4*)T.s2_P; fp.lastP = T.last_P; fp.oc = oc;
-  fp.tab = h->table_bf16 ? 1 : 0;
-  fgrid = fwd_train_grid(B, h->sm_count);
-  launch_fwd_train(NV, group, fp, fgrid, l);
+  tm.mark(FR_T_FWD);
+  // 2. forward.  (Single-pass: the norm / loss / dCat partials are complete when the kernel ends; its crossing-run combine
+  //    does not touch them: finalize runs beside the combine on a second side stream -- the event is recorded between the
+  //    two launches.  With fr_timing_enable it runs in sequence.)
+  const bool fin_aside = fused && !h->timing;
+  l.mid = fin_aside ? h->aux2_fork : nullptr;
+  const int fgrid = forward(h, r, fused, oc, l);
+  l.mid = nullptr;
   FR_CHECK_LAUNCH(h);
-  }
 
-  FR_MARK(FR_T_FINALIZE);
+  tm.mark(FR_T_FINALIZE);
   // 3. global norm -> clip scale; dense optimizer on Cat
   FinalizeParams fin{};
   fin.part_loss = h->part_loss; fin.part_nrm = h->part_nrm; fin.part_gcat = h->part_gcat; fin.nblk = fgrid;
@@ -496,8 +585,7 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   fin.oc = oc; fin.clip = h->cfg.clip_norm; fin.out = out; fin.lr_hist = h->lr_hist;
   if (fin_aside) {
     FR_CUDA(h, cudaStreamWaitEvent(h->aux2_stream, h->aux2_fork, 0));
-    Launch l2{h->sm_count, h->aux2_stream, nullptr};
-    launch_finalize(fin, l2);
+    launch_finalize(fin, Launch{h->sm_count, h->aux2_stream, nullptr});
     FR_CUDA(h, cudaEventRecord(h->aux2_join, h->aux2_stream));
     FR_CUDA(h, cudaStreamWaitEvent(st, h->aux2_join, 0));
   } else {
@@ -505,84 +593,39 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   }
   FR_CHECK_LAUNCH(h);
 
-  FR_MARK(FR_T_USER_CHUNK);
+  tm.mark(FR_T_USER_CHUNK);
   // 4. Personal_Memory: segment-reduce by user + optimizer (+ personal write)
-  {
-    l.mid = ts ? ts->ev[FR_T_USER_COMBINE] : nullptr;
-    SegCommon c = cu;
-    UserPolParams up{};
-    up.P = (float4*)T.P; up.s1 = (float4*)T.s1_P; up.s2 = (float4*)T.s2_P; up.last = T.last_P;
-    up.R = (const float4*)T.R; up.G = (const float4*)T.G; up.cat = h->cat_pre;
-    up.items = items; up.g = h->g; up.cats = cats; up.cats_by_item = cats_by_item;
-    up.ws_row = h->ws_row; up.out = out; up.group = group; up.mc = h->mc; up.oc = oc;
-    up.user_labels = b->user_labels; up.lab_off = T.user_label_off; up.lab_idx = T.user_label_idx; up.users = users;
-    up.tab = h->table_bf16 ? 1 : 0;
-    if (fused) {
-      // 4'. the norm is known.  scale == 1 exactly: the speculative rows become current (stamp bits flipped).  Otherwise
-      //     nothing was committed: every row goes back to the caller's tables and the ordinary update pass runs with
-      //     the true scale on the g / z the single-pass kernel left (both launches exit at once in the common case).
-      launch_user_commit(cu.keys, (uint32_t)S, T.last_P, out, (int)step, l);
-      launch_shadow_consolidate(T.last_P, h->cfg.num_users, 5 * DV, (float4*)T.P, (float4*)T.s1_P, (float4*)T.s2_P,
-                                (const float4*)h->shP, (const float4*)h->shM, (const float4*)h->shV, out, l);
-      c.uniq_counter = nullptr;          // (counted by the single-pass kernel)
-      c.only_if_scaled = out;
-    }
-    launch_user_pass(NV, c, up, l);
-    FR_CHECK_LAUNCH(h);
-    if (write_personal) {     // Write_Memory :149-198 on the optimizer's output; reads pre-step R, Cat, G
-      const size_t need = (size_t)S / 32 + 2;
-      if (need > h->pieces_personal_chunks) {
-        if (h->pieces_personal) { FR_CUDA(h, cudaStreamSynchronize(st)); cudaFree(h->pieces_personal); h->pieces_personal = nullptr; }
-        FR_CUDA(h, cudaMalloc(&h->pieces_personal, need * 2 * 10 * DV * sizeof(float4)));
-        h->pieces_personal_chunks = need;
-      }
-      c.pieces = h->pieces_personal;
-      c.uniq_counter = nullptr;
-      l.mid = nullptr;
-      launch_personal_pass(NV, c, up, l);
-      FR_CHECK_LAUNCH(h);
-    }
-  }
+  l.mid = tm.ev(FR_T_USER_COMBINE);
+  if ((rc = user_update(h, r, fused, write_personal, oc, step, l, nullptr))) return rc;
+  FR_CHECK_LAUNCH(h);
 
-  FR_MARK(FR_T_LABEL);
-  // 5. General_Memory: segment-reduce of the label entries (built in 1b) by label (reads pre-step R).
-  //    (Round 2 tried a shared-memory scatter with one owner warp per label instead -- no sort, no entry list: measured
-  //    354 us + 25 us against this pass's 254 us at 524k rows; see DESIGN.md "measured and rejected".)
-  {
-    l.mid = nullptr;
-    FR_CUDA(h, cudaStreamWaitEvent(st, h->aux_join, 0));      // JOIN: the side stream (entry list 1b, and the pass itself 1c)
-    if (!label_aside) { rc = label_pass(l); if (rc) return rc; }
-  }
+  tm.mark(FR_T_LABEL);
+  // 5. General_Memory (built in 1b, run in 1c on ordinary steps)
+  l.mid = nullptr;
+  FR_CUDA(h, cudaStreamWaitEvent(st, h->aux_join, 0));      // JOIN: the side stream (entry list 1b, and the pass itself 1c)
+  if (!label_aside) { label_pass(h, r, rl, l); FR_CHECK_LAUNCH(h); }
 
-  FR_MARK(FR_T_ITEM_CHUNK);
+  tm.mark(FR_T_ITEM_CHUNK);
   // 6. Recipe_Embedding: segment-reduce by recipe + optimizer
   {
-    l.mid = ts ? ts->ev[FR_T_ITEM_COMBINE] : nullptr;
+    l.mid = tm.ev(FR_T_ITEM_COMBINE);
     SegCommon c{};
     c.keys = h->sortI.k[ri]; c.perm = h->sortI.v[ri]; c.n_dev = nullptr; c.n_host = (uint32_t)S;
     c.pieces = h->pieces_i; c.uniq_counter = h->counters + 1;
     c.long_list = h->long_list; c.long_count = h->counters + 3; c.long_cap = h->long_cap;
     ItemPolParams ip{};
     ip.R = (float4*)T.R; ip.s1 = (float4*)T.s1_R; ip.s2 = (float4*)T.s2_R; ip.last = T.last_R;
-    ip.z = h->z; ip.g = h->g; ip.out = out; ip.mc = h->mc; ip.oc = oc; ip.tab = h->table_bf16 ? 1 : 0;
+    ip.z = h->z; ip.g = h->g; ip.out = out; ip.mc = h->mc; ip.oc = oc; ip.tab = tab_code(h, true);
     launch_item_pass(NV, c, ip, l);
     FR_CHECK_LAUNCH(h);
   }
 
   l.mid = nullptr;
-  FR_MARK(FR_T_SWEEP);
-  // LAZY_SERIES table: every catch-up of this step (target t-1) is done; add the s = t term so
-  // that the table serves target t (the personal-step sweep below, fr_adam_flush, step t+1)
-  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_LAZY_SERIES)
-    launch_series_update(h->cser, h->lr_hist, (int)step, h->cfg.adam_beta1, h->cfg.adam_beta2, l);
-  // 7. TF-1.x dense Adam: every untouched row decays this step too
-  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_DENSE) {
-    launch_adam_sweep((float4*)T.P, (float4*)T.s1_P, (float4*)T.s2_P, T.last_P, h->cfg.num_users, 5 * DV, oc, (int)step, l);
-    launch_adam_sweep((float4*)T.R, (float4*)T.s1_R, (float4*)T.s2_R, T.last_R, h->cfg.num_items, DV, oc, (int)step, l);
-    FR_CHECK_LAUNCH(h);
-  }
+  tm.mark(FR_T_SWEEP);
+  optimizer_tail(h, oc, step, l);
+  FR_CHECK_LAUNCH(h);
 
-  FR_MARK(FR_T_MISC);
+  tm.mark(FR_T_MISC);
   // 8. fetches: general = mean(G) (:219), personal = mean(P) (:218, personal steps only)
   if (!label_aside)
     launch_mean((const float4*)T.G, (int64_t)h->mc.L * 5 * DV, h->mean_partials, out + FR_OUT_GENERAL,
@@ -597,12 +640,8 @@ extern "C" int fr_train_step(fr_handle h, const fr_batch* b, int32_t write_perso
   }
   launch_write_counters(h->counters, out, l);
   FR_CHECK_LAUNCH(h);
-  FR_MARK(FR_T_COUNT);
-#undef FR_MARK
-
-  h->step = step;
-  h->b1p *= h->cfg.adam_beta1;     // adam.py _finish
-  h->b2p *= h->cfg.adam_beta2;
+  tm.mark(FR_T_COUNT);
+  step_advance(h, step);
   return FR_OK;
 }
 
@@ -690,39 +729,19 @@ extern "C" int fr_train_step_host(fr_handle h, const fr_batch* hb, int32_t write
       return FR_OK;
     }
   }
-  const int group = hb->mode == FR_BPR ? 2 : 1;
-  const int B = hb->n_groups;
-  if (B <= 0) return fail(h, FR_ERR_ARG, "empty batch");
-  const size_t S = (size_t)B * group, L = (size_t)h->mc.L;
+  if (hb->n_groups <= 0) return fail(h, FR_ERR_ARG, "empty batch");
   cudaStream_t st = (cudaStream_t)s;
-  auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-  const size_t o_users = 0;
-  const size_t o_items = o_users + al(B * 4);
-  const size_t o_cats = o_items + al(S * 4);
-  const size_t o_labels = o_cats + al(hb->cats ? S * 16 : 0);
-  const size_t o_ws = o_labels + al(hb->labels ? (size_t)B * 4 : 0);
-  const size_t o_ul = o_ws + al(hb->write_sign ? S * 4 : 0);
-  const size_t o_out = o_ul + al(hb->user_labels ? (size_t)B * L * 4 : 0);
-  const size_t total = o_out + al(FR_OUT_COUNT * 4);
-  if (total > h->stage_bytes) {
+  const FeedLayout f = feed_layout(h, hb);
+  if (f.total > h->stage_bytes) {
     if (h->stage) { FR_CUDA(h, cudaStreamSynchronize(st)); cudaFree(h->stage); h->stage = nullptr; }
-    FR_CUDA(h, cudaMalloc(&h->stage, total));
-    h->stage_bytes = total;
+    FR_CUDA(h, cudaMalloc(&h->stage, f.total));
+    h->stage_bytes = f.total;
   }
-  char* base = (char*)h->stage;
-  fr_batch db = *hb;
-#define H2D(field, off, bytes) if (hb->field) { \
-    FR_CUDA(h, cudaMemcpyAsync(base + (off), hb->field, (bytes), cudaMemcpyHostToDevice, st)); \
-    db.field = reinterpret_cast<decltype(db.field)>(base + (off)); }
-  H2D(users, o_users, (size_t)B * 4)
-  H2D(items, o_items, S * 4)
-  H2D(cats, o_cats, S * 16)
-  H2D(labels, o_labels, (size_t)B * 4)
-  H2D(write_sign, o_ws, S * 4)
-  H2D(user_labels, o_ul, (size_t)B * L * 4)
-#undef H2D
-  float* dout = reinterpret_cast<float*>(base + o_out);
-  int rc = fr_train_step(h, &db, write_personal, dout, nullptr, s);
+  fr_batch db;
+  int rc = feed_copy(h, hb, f, static_cast<char*>(h->stage), &db, st);
+  if (rc) return rc;
+  float* dout = reinterpret_cast<float*>(static_cast<char*>(h->stage) + f.out);
+  rc = fr_train_step(h, &db, write_personal, dout, nullptr, s);
   if (rc) return rc;
   if (host_out_scalars)
     FR_CUDA(h, cudaMemcpyAsync(host_out_scalars, dout, FR_OUT_COUNT * sizeof(float), cudaMemcpyDeviceToHost, st));

@@ -266,6 +266,19 @@ extern "C" int fr_shard_serve(fr_handle h, const fr_shard* sh, const int32_t* rr
 }
 
 // ---------------------------------------------------------------- 3. forward
+// The rows of this rank's step (plan slot ps), read from the received recipe rows
+static StepRows shard_rows(fr_ctx* h, const fr_ctx::PlanSlot& ps, const fr_batch* b, const fr_shard* sh, const float* rbuf,
+                           float* out, float* dG) {
+  StepRows r{};
+  r.B = ps.B; r.S = ps.S; r.group = ps.group;
+  r.users = ps.users_s; r.items = ps.slot_of_row; r.ws_row = ps.ws_row;
+  r.ukeys = ps.sortU.k[ps.ru]; r.uperm = ps.sortU.v[ps.ru];
+  r.R = (const float4*)rbuf; r.R_is_table = false; r.cats = ps.cats_row; r.cats_by_item = 0;
+  r.labels = b->labels; r.user_labels = b->user_labels; r.Bnorm = (float)sh->global_batch;
+  r.out = out; r.scores = h->scores; r.G = (float4*)dG;
+  return r;
+}
+
 extern "C" int fr_shard_forward(fr_handle h, const fr_batch* b, const fr_shard* sh, const float* rbuf, float* packed,
                                 fr_stream s) {
   int rc = shard_check(h, sh); if (rc) return rc;
@@ -283,93 +296,31 @@ extern "C" int fr_shard_forward(fr_handle h, const fr_batch* b, const fr_shard* 
   // pre-step snapshot of Category_Embedding (every read of Cat in this step sees it)
   FR_CUDA(h, cudaMemcpyAsync(h->cat_pre, h->tab.Cat, (size_t)4 * h->mc.D * sizeof(float), cudaMemcpyDeviceToDevice, st));
   Launch l{h->sm_count, st, nullptr};
-  const fr_tables& T = h->tab;
-  const int DV = h->mc.DV, NV = h->NV, S = ps.S, B = ps.B;
   const OptConsts oc = make_oc(h, h->step + 1);
-  const bool lazy = h->cfg.learner == FR_ADAM && h->cfg.adam_mode != FR_ADAM_DENSE;
+  const StepRows r = shard_rows(h, ps, b, sh, rbuf, ps.flag_out, packed + 4 + 4 * (size_t)h->mc.D);
 
-  const bool aside = !getenv("FOODREC_LABEL_SERIAL");
-  auto label_chain = [&](Launch& la) -> int {
-    // General_Memory delta of this rank's rows -> packed (G itself is updated after the all-reduce).  Entry list (count,
-    // scan, emit, sort by label) and the segment reduce read only the batch, the received rows and the Cat snapshot: they
-    // run on the library's side stream BESIDE the forward / single-pass kernel (bandwidth-bound; this chain is issue- and
-    // latency-bound) and are joined at the end of the phase (FOODREC_LABEL_SERIAL: in sequence, as before).
-    float* dG = packed + 4 + 4 * (size_t)h->mc.D;
-    FR_CUDA(h, cudaMemsetAsync(dG, 0, 5 * (size_t)h->mc.L * h->mc.D * sizeof(float), la.st));
-    LabelEmitParams ep{};
-    ep.S = S; ep.group = ps.group; ep.L = h->mc.L; ep.users = ps.users_s;
-    ep.user_labels = b->user_labels; ep.lab_off = T.user_label_off; ep.lab_idx = T.user_label_idx;
-    ep.ws_row = ps.ws_row; ep.counts = h->counts; ep.offs = h->offs;
-    ep.ent_key = h->ent_key; ep.ent_row = h->ent_row; ep.ent_coef = h->ent_coef;
-    ep.cap = (uint32_t)h->sortL.cap; ep.n_entries = h->n_entries; ep.out = ps.flag_out;
-    launch_label_count(ep, la);
-    exclusive_scan_u32(h->counts, h->offs, (uint32_t)S, h->scan_tmp, h->n_entries, la.st);
-    launch_label_emit(ep, la);
-    const uint32_t ecap = (uint32_t)h->sortL.cap;
-    const int rl = radix_sort_pairs(h->sortL, h->ent_key, ecap, h->n_entries, bits_for(h->mc.L), la.st, h->sm_count);
-    SegCommon c{};
-    c.keys = h->sortL.k[rl]; c.perm = h->sortL.v[rl]; c.n_dev = h->n_entries; c.n_host = ecap;
-    c.pieces = h->pieces_g; c.uniq_counter = nullptr;
-    c.long_list = h->long_list; c.long_count = h->counters + 2; c.long_cap = h->long_cap;
-    LabelPolParams lp{};
-    lp.G = (float4*)dG; lp.R = (const float4*)rbuf; lp.cat = h->cat_pre;
-    lp.ent_row = h->ent_row; lp.ent_coef = h->ent_coef; lp.items = ps.slot_of_row; lp.cats = ps.cats_row;
-    lp.cats_by_item = 0; lp.mc = h->mc; lp.tab = 0;
-    launch_label_pass(NV, c, lp, la);
-    FR_CHECK_LAUNCH(h);
-    return FR_OK;
-  };
-  if (aside) {
-    if ((rc = aux_ensure(h))) return rc;
-    FR_CUDA(h, cudaEventRecord(h->aux_fork, st));
-    FR_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->aux_fork, 0));
-    Launch la{h->sm_count, h->aux_stream, nullptr};
-    rc = label_chain(la); if (rc) return rc;
-    FR_CUDA(h, cudaEventRecord(h->aux_join, h->aux_stream));
-  }
+  // General_Memory delta of this rank's rows -> packed (G itself is updated after the all-reduce).  Entry list and segment
+  // reduce read only the batch, the received rows and the Cat snapshot: they run on the library's side stream BESIDE the
+  // forward / single-pass kernel (bandwidth-bound; this chain is issue- and latency-bound), joined at the end of the phase.
+  if ((rc = aux_ensure(h))) return rc;
+  FR_CUDA(h, cudaEventRecord(h->aux_fork, st));
+  FR_CUDA(h, cudaStreamWaitEvent(h->aux_stream, h->aux_fork, 0));
+  const Launch la{h->sm_count, h->aux_stream, nullptr};
+  FR_CUDA(h, cudaMemsetAsync(r.G, 0, 5 * (size_t)h->mc.L * h->mc.D * sizeof(float), la.st));
+  label_pass(h, r, label_entries(h, r, la), la);
+  FR_CHECK_LAUNCH(h);
+  FR_CUDA(h, cudaEventRecord(h->aux_join, h->aux_stream));
 
-  int fgrid;
-  ps.fused = lazy && h->shP && !getenv("FOODREC_TWO_PASS");
-  if (ps.fused) {
-    // single-pass step (train_seg.cu): forward AND the speculative Personal_Memory update, before the all-reduce that
-    // makes the global norm known; fr_shard_update commits the rows (scale == 1) or redoes the update with the true scale
-    SegCommon cu{};
-    cu.keys = ps.sortU.k[ps.ru]; cu.perm = ps.sortU.v[ps.ru]; cu.n_dev = nullptr; cu.n_host = (uint32_t)S;
-    cu.uniq_counter = h->counters + 0; cu.pieces = h->pieces_u;
-    FusedParams fz{};
-    fz.P[0] = (float4*)T.P; fz.m[0] = (float4*)T.s1_P; fz.v[0] = (float4*)T.s2_P;
-    fz.P[1] = (float4*)h->shP; fz.m[1] = (float4*)h->shM; fz.v[1] = (float4*)h->shV;
-    fz.last = T.last_P; fz.R = (const float4*)rbuf; fz.cat = h->cat_pre;
-    fz.items = ps.slot_of_row; fz.cats = ps.cats_row; fz.cats_by_item = 0; fz.labels = b->labels;
-    fz.a = h->mc.a; fz.oma = h->mc.oma; fz.Bnorm = (float)sh->global_batch;
-    fz.g = h->g; fz.z = h->z; fz.scores = h->scores;
-    fz.part_loss = h->part_loss; fz.part_nrm = h->part_nrm; fz.part_gcat = h->part_gcat;
-    fz.mc = h->mc; fz.oc = oc;
-    fgrid = user_fused_grid((uint32_t)S, h->sm_count);
-    launch_user_fused(NV, ps.group, cu, fz, fgrid, l);
-    h->shadow_dirty = true;
-  } else {
-  FwdParams fp{};
-  fp.P = (const float4*)T.P; fp.R = (const float4*)rbuf; fp.cat = h->cat_pre; fp.DV = DV; fp.B = B;
-  fp.Bnorm = (float)sh->global_batch;
-  fp.users = ps.users_s; fp.items = ps.slot_of_row; fp.cats = ps.cats_row; fp.cats_by_item = 0;
-  fp.labels = b->labels; fp.a = h->mc.a; fp.oma = h->mc.oma;
-  fp.g = h->g; fp.z = h->z; fp.scores = h->scores;
-  fp.part_loss = h->part_loss; fp.part_nrm = h->part_nrm; fp.part_gcat = h->part_gcat;
-  fp.lazy = lazy ? 1 : 0; fp.mP = (const float4*)T.s1_P; fp.vP = (const float4*)T.s2_P; fp.lastP = T.last_P; fp.oc = oc;
-  fp.tab = h->table_bf16 ? 2 : 0;        // bf16 Personal_Memory, fp32 received recipe rows
-  fgrid = fwd_train_grid(B, h->sm_count);
-  launch_fwd_train(NV, ps.group, fp, fgrid, l);
-  }
-
+  // single-pass: forward AND the speculative Personal_Memory update, before the all-reduce that makes the global norm
+  // known; fr_shard_update commits the rows (scale == 1) or redoes the update with the true scale
+  ps.fused = single_pass(h);
+  const int fgrid = forward(h, r, ps.fused, oc, l);
   FinalizeParams fin{};
   fin.part_loss = h->part_loss; fin.part_nrm = h->part_nrm; fin.part_gcat = h->part_gcat; fin.nblk = fgrid;
-  fin.DV = DV; fin.B = (float)sh->global_batch; fin.packed = packed; fin.do_reduce = 1; fin.do_apply = 0;
+  fin.DV = h->mc.DV; fin.B = r.Bnorm; fin.packed = packed; fin.do_reduce = 1; fin.do_apply = 0;
   fin.oc = oc; fin.clip = h->cfg.clip_norm; fin.out = ps.flag_out; fin.lr_hist = nullptr;
   launch_finalize(fin, l);
-
-  if (aside) FR_CUDA(h, cudaStreamWaitEvent(st, h->aux_join, 0));
-  else { rc = label_chain(l); if (rc) return rc; }
+  FR_CUDA(h, cudaStreamWaitEvent(st, h->aux_join, 0));
   FR_CHECK_LAUNCH(h);
   return FR_OK;
 }
@@ -394,61 +345,23 @@ extern "C" int fr_shard_update(fr_handle h, const fr_batch* b, const fr_shard* s
   float* out = out_scalars ? out_scalars : ps.flag_out;
   if (out != ps.flag_out)   // flags raised by plan/forward (capacity / label overflow / id range)
     FR_CUDA(h, cudaMemcpyAsync(out, ps.flag_out, FR_OUT_COUNT * sizeof(float), cudaMemcpyDeviceToDevice, st));
+  const StepRows r = shard_rows(h, ps, b, sh, rbuf, out, nullptr);
 
   // fr_timing_*: the events of this phase's kernels (user pass, personal pass + dG add as "label", local recipe-gradient
   // pass); the phases that live in other fr_shard_* calls read as zero
-  fr_ctx::TimingSet* ts = nullptr;
-  if (h->timing) {
-    ts = &h->tsets[h->ts_next++ % h->tsets.size()];
-    timing_collect(h, *ts);
-    ts->used = true;
-  }
-#define FR_MARK(i) do { if (ts) cudaEventRecord(ts->ev[i], st); } while (0)
-  FR_MARK(FR_T_SORT); FR_MARK(FR_T_FWD); FR_MARK(FR_T_FINALIZE);
+  const StepTiming tm(h, st);
+  tm.mark(FR_T_SORT); tm.mark(FR_T_FWD); tm.mark(FR_T_FINALIZE);
   FinalizeParams fin{};
-  fin.DV = DV; fin.B = (float)sh->global_batch; fin.packed = const_cast<float*>(packed_reduced);
+  fin.DV = DV; fin.B = r.Bnorm; fin.packed = const_cast<float*>(packed_reduced);
   fin.do_reduce = 0; fin.do_apply = 1;
   fin.Cat = (float4*)T.Cat; fin.s1Cat = (float4*)T.s1_Cat; fin.s2Cat = (float4*)T.s2_Cat;
   fin.oc = oc; fin.clip = h->cfg.clip_norm; fin.out = out; fin.lr_hist = h->lr_hist;
   launch_finalize(fin, l);
 
-  SegCommon c{};
-  c.keys = ps.sortU.k[ps.ru]; c.perm = ps.sortU.v[ps.ru]; c.n_dev = nullptr; c.n_host = (uint32_t)S;
-  c.uniq_counter = h->counters + 0; c.pieces = h->pieces_u;
-  UserPolParams up{};
-  up.P = (float4*)T.P; up.s1 = (float4*)T.s1_P; up.s2 = (float4*)T.s2_P; up.last = T.last_P;
-  up.R = (const float4*)rbuf; up.G = (const float4*)T.G; up.cat = h->cat_pre;
-  up.items = ps.slot_of_row; up.g = h->g; up.cats = ps.cats_row; up.cats_by_item = 0;
-  up.ws_row = ps.ws_row; up.out = out; up.group = ps.group; up.mc = h->mc; up.oc = oc;
-  up.user_labels = b->user_labels; up.lab_off = T.user_label_off; up.lab_idx = T.user_label_idx; up.users = ps.users_s;
-  up.tab = h->table_bf16 ? 2 : 0;
-  FR_MARK(FR_T_USER_CHUNK);
-  l.mid = ts ? ts->ev[FR_T_USER_COMBINE] : nullptr;
-  if (S > 0 && ps.fused) {
-    // the all-reduce made the norm known: commit the speculative rows (scale == 1), else bring every row back to the
-    // caller's tables and run the ordinary update pass with the true scale (both exit at once in the common case)
-    launch_user_commit(c.keys, (uint32_t)S, T.last_P, out, (int)step, l);
-    launch_shadow_consolidate(T.last_P, h->cfg.num_users, 5 * DV, (float4*)T.P, (float4*)T.s1_P, (float4*)T.s2_P,
-                              (const float4*)h->shP, (const float4*)h->shM, (const float4*)h->shV, out, l);
-    c.uniq_counter = nullptr;
-    c.only_if_scaled = out;
-  }
-  if (S > 0) launch_user_pass(NV, c, up, l);
-  else if (l.mid) cudaEventRecord(l.mid, st);
+  tm.mark(FR_T_USER_CHUNK);
+  l.mid = tm.ev(FR_T_USER_COMBINE);
+  if ((rc = user_update(h, r, ps.fused, write_personal, oc, step, l, tm.ev(FR_T_LABEL)))) return rc;
   l.mid = nullptr;
-  FR_MARK(FR_T_LABEL);
-  if (write_personal && S > 0) {
-    if (ps.fused) { rc = shadow_sync(h, st); if (rc) return rc; }     // the personal pass works on the caller's table
-    c.only_if_scaled = nullptr;                                      // (it always runs, whatever the clip did)
-    const size_t need = (size_t)S / 32 + 2;
-    if (need > h->pieces_personal_chunks) {
-      if (h->pieces_personal) { FR_CUDA(h, cudaStreamSynchronize(st)); cudaFree(h->pieces_personal); h->pieces_personal = nullptr; }
-      FR_CUDA(h, cudaMalloc(&h->pieces_personal, need * 2 * 10 * DV * sizeof(float4)));
-      h->pieces_personal_chunks = need;
-    }
-    c.pieces = h->pieces_personal; c.uniq_counter = nullptr;
-    launch_personal_pass(NV, c, up, l);
-  }
   // G += all-reduced delta (after the personal pass, which reads G_old)
   launch_add_inplace((float4*)T.G, (const float4*)(packed_reduced + 4 + 4 * (size_t)h->mc.D), (int64_t)h->mc.L * 5 * DV, l);
 
@@ -460,13 +373,12 @@ extern "C" int fr_shard_update(fr_handle h, const fr_batch* b, const fr_shard* s
   ItemPolParams ip{};
   ip.z = h->z; ip.g = h->g; ip.out = out; ip.mc = h->mc; ip.oc = oc;
   PeerPtrs none{}; none.world = 0;
-  FR_MARK(FR_T_ITEM_CHUNK);
-  l.mid = ts ? ts->ev[FR_T_ITEM_COMBINE] : nullptr;
+  tm.mark(FR_T_ITEM_CHUNK);
+  l.mid = tm.ev(FR_T_ITEM_COMBINE);
   if (S > 0) launch_item_grad_pass(NV, ci, ip, (float4*)grows, grows ? none : w.peer_rgrows, l);
   else if (l.mid) cudaEventRecord(l.mid, st);
   l.mid = nullptr;
-  FR_MARK(FR_T_SWEEP); FR_MARK(FR_T_MISC); FR_MARK(FR_T_COUNT);
-#undef FR_MARK
+  tm.mark(FR_T_SWEEP); tm.mark(FR_T_MISC); tm.mark(FR_T_COUNT);
   FR_CHECK_LAUNCH(h);
   return FR_OK;
 }
@@ -496,15 +408,9 @@ extern "C" int fr_shard_apply(fr_handle h, const fr_shard* sh, const int32_t* rr
   c.pieces = w.pieces_s; c.uniq_counter = nullptr;
   ItemPolParams ip{};
   ip.R = (float4*)T.R; ip.s1 = (float4*)T.s1_R; ip.s2 = (float4*)T.s2_R; ip.last = T.last_R;
-  ip.z = (const float4*)rgrows; ip.g = nullptr; ip.out = out; ip.mc = h->mc; ip.oc = oc; ip.tab = h->table_bf16 ? 1 : 0;
+  ip.z = (const float4*)rgrows; ip.g = nullptr; ip.out = out; ip.mc = h->mc; ip.oc = oc; ip.tab = tab_code(h, true);
   launch_item_pass(NV, c, ip, l);
-
-  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_LAZY_SERIES)
-    launch_series_update(h->cser, h->lr_hist, (int)step, h->cfg.adam_beta1, h->cfg.adam_beta2, l);
-  if (h->cfg.learner == FR_ADAM && h->cfg.adam_mode == FR_ADAM_DENSE) {
-    launch_adam_sweep((float4*)T.P, (float4*)T.s1_P, (float4*)T.s2_P, T.last_P, h->cfg.num_users, 5 * DV, oc, (int)step, l);
-    launch_adam_sweep((float4*)T.R, (float4*)T.s1_R, (float4*)T.s2_R, T.last_R, h->cfg.num_items, DV, oc, (int)step, l);
-  }
+  optimizer_tail(h, oc, step, l);
   launch_mean((const float4*)T.G, (int64_t)h->mc.L * 5 * DV, h->mean_partials, out + FR_OUT_GENERAL,
               (double)h->mc.L * 5.0 * h->mc.D, l);
   launch_write_counters(h->counters, out, l);
@@ -512,8 +418,6 @@ extern "C" int fr_shard_apply(fr_handle h, const fr_shard* sh, const int32_t* rr
   ps.S = 0; ps.planned = false;
   sv.prepared = false;
   ++w.n_apply;
-  h->step = step;
-  h->b1p *= h->cfg.adam_beta1;
-  h->b2p *= h->cfg.adam_beta2;
+  step_advance(h, step);
   return FR_OK;
 }

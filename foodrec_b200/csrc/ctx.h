@@ -130,6 +130,36 @@ static inline void timing_collect(fr_ctx* h, fr_ctx::TimingSet& ts) {
   ts.used = false;
 }
 
+// The phase events of one step on stream st (fr_timing_*); every call is a no-op while timing is off
+struct StepTiming {
+  fr_ctx::TimingSet* ts = nullptr;
+  cudaStream_t st;
+  StepTiming(fr_ctx* h, cudaStream_t s) : st(s) {
+    if (!h->timing) return;
+    ts = &h->tsets[h->ts_next++ % h->tsets.size()];
+    timing_collect(h, *ts);
+    ts->used = true;
+  }
+  void mark(int i) const { if (ts) cudaEventRecord(ts->ev[i], st); }
+  cudaEvent_t ev(int i) const { return ts ? ts->ev[i] : nullptr; }
+};
+
+// Where the rows of a training step come from: the single-GPU step reads the tables, the row-sharded phases the rows
+// this rank planned and received.  The phase builders below take everything else from the context.
+struct StepRows {
+  int B, S, group;
+  const int32_t *users, *items;       // range-checked user rows; each row's recipe row in R
+  const float* ws_row;                // write sign of each row
+  const uint32_t *ukeys, *uperm;      // the rows sorted by user: keys, permutation
+  const float4* R; bool R_is_table;   // the recipe rows read: Recipe_Embedding, or the received rows (always fp32)
+  const float4* cats; int cats_by_item;
+  const float *labels, *user_labels;  // the batch's
+  float Bnorm;                        // divisor of the loss mean: the (global) batch size
+  float* out;                         // flags and scalars
+  float* scores;
+  float4* G;                          // target of the label pass: General_Memory, or this rank's delta of it
+};
+
 static inline int fail(fr_ctx* h, int code, const char* fmt, ...) {
   if (h) {
     va_list ap; va_start(ap, fmt);
@@ -201,3 +231,13 @@ int ensure_lr_hist(fr_ctx* h, int64_t need, cudaStream_t st);
 int shadow_sync(fr_ctx* h, cudaStream_t st);     // rows whose current copy is the shadow go back to the caller's tables
 float adam_lr_t(const fr_ctx* h);
 fr::OptConsts make_oc(const fr_ctx* h, int64_t step);
+// Phases of a training step, shared by fr_train_step and the row-sharded phases (api.cu)
+bool single_pass(const fr_ctx* h);              // the step runs the single-pass kernel (lazy Adam, fr_set_shadow)
+int tab_code(const fr_ctx* h, bool R_is_table);  // FwdParams::tab
+int label_entries(fr_ctx* h, const StepRows& r, const Launch& l);   // label entry list, sorted; returns the sort's result
+void label_pass(fr_ctx* h, const StepRows& r, int rl, const Launch& l);
+int forward(fr_ctx* h, const StepRows& r, bool fused, const fr::OptConsts& oc, const Launch& l);   // returns its grid
+int user_update(fr_ctx* h, const StepRows& r, bool fused, bool write_personal, const fr::OptConsts& oc, int64_t step,
+                Launch l, cudaEvent_t before_personal);
+void optimizer_tail(fr_ctx* h, const fr::OptConsts& oc, int64_t step, const Launch& l);
+void step_advance(fr_ctx* h, int64_t step);
