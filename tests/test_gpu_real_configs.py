@@ -16,6 +16,7 @@ import torch
 
 from oracle import synth
 from oracle.recommender_oracle import Hyper as OHyper, OracleModel
+from tests.test_adam_strict_regime import regime_guard, report
 from tests.util import assert_close, assert_close_adam
 
 pytestmark = pytest.mark.gpu
@@ -105,8 +106,10 @@ def _bpr_batches(B, steps, seed):
     return out
 
 
-def _run_cfg2(configs, B, steps, seed):
-    """configs: list of (learner, adam_mode, lr) that share ONE oracle run (same learner, same lr)."""
+def _run_cfg2(configs, B, steps, seed, adam_eps=1e-8, strict=False):
+    """configs: list of (learner, adam_mode, lr) that share ONE oracle run (same learner, same lr).  strict (Adam): every
+    touched entry is held to the plain 1e-5 rule, after the regime guard of tests/test_adam_strict_regime.py has checked
+    that adam_eps keeps the quotient well conditioned for these gradients."""
     from foodrec_b200 import Engine, Hyper, _lib as L
     dev = torch.device("cuda:0")
     learner, lr = configs[0][0], configs[0][2]
@@ -124,10 +127,11 @@ def _run_cfg2(configs, B, steps, seed):
     su0 = P.view(torch.int32)[mu].to(torch.int64).sum().item()
     si0 = R.view(torch.int32)[mi].to(torch.int64).sum().item()
 
-    om = OracleModel(P0c, R0c, Cat0, G0, OHyper(learner=learner, lr=lr), dtype=np.float64)
-    om32 = OracleModel(P0c, R0c, Cat0, G0, OHyper(learner=learner, lr=lr), dtype=np.float32) if learner == "adam" else None
-    engines = [Engine(Hyper(learner=learner, lr=lr), P.clone(), R.clone(), Cat.clone(), G.clone(), device=dev, max_rows=2 * B,
-                      adam_mode=mode, item_cats=ic, user_label_csr=lab, adopt=True) for _, mode, _ in configs]
+    om = OracleModel(P0c, R0c, Cat0, G0, OHyper(learner=learner, lr=lr, adam_eps=adam_eps), dtype=np.float64)
+    om32 = OracleModel(P0c, R0c, Cat0, G0, OHyper(learner=learner, lr=lr, adam_eps=adam_eps),
+                       dtype=np.float32) if learner == "adam" else None
+    engines = [Engine(Hyper(learner=learner, lr=lr, adam_eps=adam_eps), P.clone(), R.clone(), Cat.clone(), G.clone(),
+                      device=dev, max_rows=2 * B, adam_mode=mode, item_cats=ic, user_label_csr=lab, adopt=True) for _, mode, _ in configs]
     del P, R
     for users, pos, neg in bs:
         f = dict(user_input=np.searchsorted(uu, users), item_input=np.searchsorted(ui, pos),
@@ -145,15 +149,19 @@ def _run_cfg2(configs, B, steps, seed):
             assert v[1] == pytest.approx(o["norm"], rel=1e-5)
             assert v[2] == 1.0 and o["scale"] == 1.0                 # (the clip is inactive at this batch size)
             assert int(v[6]) == len(np.unique(users)) and int(v[7]) == len(np.unique(np.concatenate([pos, neg])))
+    if strict:
+        regime_guard(om, om32, f"cfg2 B={B} adam_eps={adam_eps:g}")
     for (lrn, mode, _), e in zip(configs, engines):
         e.flush()
         got = {"P": e.P[tu].cpu().numpy(), "R": e.R[ti].cpu().numpy(), "Cat": e.Cat.cpu().numpy(), "G": e.G.cpu().numpy()}
         for k in ("P", "R", "Cat", "G"):
             what = f"cfg2 B={B} {lrn}/{mode} {k}"
-            if om32 is not None and k != "G":
+            if om32 is not None and k != "G" and not strict:
                 assert_close_adam(got[k], getattr(om, k), getattr(om32, k), what=what)
             else:
                 assert_close(got[k], getattr(om, k), what=what)
+        if strict:
+            report(got, om, f"cfg2 B={B} {lrn}/{mode} adam_eps={adam_eps:g}")
         assert e.P.view(torch.int32)[mu].to(torch.int64).sum().item() == su0, "an untouched Personal_Memory row changed"
         assert e.R.view(torch.int32)[mi].to(torch.int64).sum().item() == si0, "an untouched Recipe_Embedding row changed"
         e.close()
