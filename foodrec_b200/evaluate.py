@@ -12,7 +12,8 @@ scoring, dict-dedup and the stable top-K in one launch.  HR / NDCG use the same 
 against EVERY recipe the user did not train on, through the full-catalog top-K with the user's
 training items excluded.
 
-``evaluate_sharded`` is ``evaluate_model`` on row-sharded tables (``sharded.DistRunner`` / ``LocalRunner``).
+``evaluate_sharded`` is ``evaluate_model`` on row-sharded tables (``sharded.DistRunner`` / ``LocalRunner``), and
+``evaluate_full_catalog_sharded`` is ``evaluate_full_catalog`` on them.
 """
 from __future__ import annotations
 
@@ -104,4 +105,47 @@ def evaluate_full_catalog(sess, model, trainMatrix, testRatings, K, dish_to_cate
         pos = np.nonzero(ids[r] == h)[0]
         hits.append(1 if pos.size else 0)                                         # getHitRatio :69-73
         ndcgs.append(math.log(2) / math.log(int(pos[0]) + 2) if pos.size else 0)  # getNDCG :76-81
+    return hits, ndcgs
+
+
+def evaluate_full_catalog_sharded(runner, trainMatrix, testRatings, K, round_users=None):
+    """``evaluate_full_catalog`` on row-sharded tables: ``runner`` is a ``sharded.LocalRunner`` or a
+    ``sharded.DistRunner`` (every rank passes the same ``trainMatrix`` / ``testRatings``).  ``trainMatrix`` is the
+    reference's dict or a global ``(offsets, ids)`` CSR over all users; each rank keeps its users' rows and hands them to
+    the runner's ``full_ranking`` (a history set for sampling stays as it is).  Each test user is ranked by its owner
+    (user % W) against every recipe with a category (the engines' ``item_cats_global``) it did not train on, the held-out
+    recipe ``testRatings[u][0]`` kept; every rank gets all users' hits and NDCGs in ``testRatings`` order."""
+    import torch
+    from .engine import history_csr
+    from .sharded import shard_label_csr
+    users, held = [], []
+    for user in testRatings:
+        if len(testRatings[str(user)]) == 0:
+            raise ValueError(f"user {user} has no test rating (evaluate.py:37 would return None and crash :29)")
+        users.append(int(user)); held.append(int(testRatings[str(user)][0]))
+    users, held = np.asarray(users, np.int64), np.asarray(held, np.int64)
+    kw = {} if round_users is None else {"round_users": int(round_users)}
+    local = hasattr(runner, "engs")
+    g0 = runner.engs[0] if local else runner.eng
+    W = g0.world
+    n_users = g0.U_global if g0.U_global is not None else g0.e.U * W
+    off, ids = history_csr(trainMatrix, n_users)
+    owner = users % W
+    per = [np.nonzero(owner == r)[0] for r in range(W)]
+    pos = np.empty(len(users), np.int64)
+    if local:
+        outs = runner.full_ranking([users[ix] // W for ix in per], [held[ix] for ix in per], K,
+                                   history=[shard_label_csr(off, ids, r, W, n_users) for r in range(W)], **kw)
+        for ix, p in zip(per, outs):
+            pos[ix] = p.cpu().numpy()
+    else:
+        r = runner.eng.rank
+        ix = per[r]
+        p = runner.full_ranking(users[ix] // W, held[ix], K, history=shard_label_csr(off, ids, r, W, n_users), **kw)
+        full = torch.zeros(len(users), dtype=torch.int32, device=p.device)     # position + 1 at this rank's users
+        full[torch.as_tensor(ix, dtype=torch.int64, device=p.device)] = p + 1
+        runner.dist.all_reduce(full)
+        pos[:] = full.cpu().numpy().astype(np.int64) - 1
+    hits = [1 if r >= 0 else 0 for r in pos]                                   # getHitRatio :69-73
+    ndcgs = [math.log(2) / math.log(int(r) + 2) if r >= 0 else 0 for r in pos]  # getNDCG :76-81
     return hits, ndcgs

@@ -26,6 +26,10 @@ from .engine import Engine, Hyper, _ptr, exclusion_csr, history_csr
 # W * cap rows, cap ~ 1.25 * round_users * stride / W: at 65,536 users x 51 candidates and D = 128, 2.1 GB of fp32 rows
 # each at W = 8, at most 1.7 GB at W = 1 (cap is also bounded by the rows an owner holds)
 EVAL_ROUND_USERS = 65536
+# test users per round of the sharded full-ranking evaluation.  A round is one catalog_topk call: every rank holds the
+# W * round_users gathered query rows (5*D fp32: 1.3 GB at W = 8, D = 128), the gathered exclusion lists and W *
+# round_users lists of K (int32 id, fp64 score) per recipe shard
+FULL_RANKING_ROUND_USERS = 65536
 
 
 # ---------------------------------------------------------------------------- host-side layout
@@ -616,6 +620,29 @@ class DistRunner:
         _eval_check_flag(flag)
         return (ids, rank, sc) if return_scores else (ids, rank)
 
+    def full_ranking(self, users_local, held_out_global, K, history=None, round_users=FULL_RANKING_ROUND_USERS):
+        """Full-ranking evaluation of this rank's test users (LOCAL rows) on the row-sharded tables: int32 [n] on the
+        device, the 0-based position of each user's held-out recipe (GLOBAL id) in its top K of the whole catalog
+        without the user's training recipes, or -1.  A user's list is its row of ``history`` (this rank's local
+        ``(offsets, ids)`` CSR, ``shard_label_csr``; None: the one ``ShardedEngine.set_user_history`` set) with every
+        occurrence of the held-out recipe removed, as ``evaluate_full_catalog`` does.  Users go in rounds of
+        ``round_users``, each one ``catalog_topk`` call; every rank walks the same rounds (one all-reduce agrees on
+        their number and on the errors: a test user outside the shard's rows that hold one, or a rank without a
+        history, raises on every rank), a rank out of users pads with local row 0 and empty lists."""
+        d, g = self.dist, self.eng
+        u, h, hist, flags = _full_ranking_inputs(g, users_local, held_out_global, history)
+        d.all_reduce(flags, op=d.ReduceOp.MAX)
+        n_max = _full_ranking_check(flags)
+        n = u.numel()
+        rn = max(1, min(int(round_users), n_max))
+        pos = torch.full((n,), -1, dtype=torch.int32, device=u.device)
+        for a in range(0, n_max, rn):
+            lo, hi = min(a, n), min(a + rn, n)
+            uu, excl = _round_lists(u, h, hist, lo, hi, rn)
+            ids, _ = self.catalog_topk(uu, K, exclude=excl)
+            pos[lo:hi] = _positions(ids[:hi - lo], h[lo:hi])
+        return pos
+
     def _gather_exclusion(self, exclude, n, dev):
         """This rank's lists for its n query rows -> the CSR of all W*n gathered rows (rank order)."""
         d, W = self.dist, self.eng.world
@@ -644,6 +671,65 @@ def _eval_check_flag(flag):
     if float(flag.max()) != 0:
         raise L.FoodRecError("sharded evaluation: a rank needed more distinct recipes from one owner than the per-owner "
                              "capacity of a round; raise cap= or lower round_users=")
+
+
+def _full_ranking_inputs(g, users_local, held_out_global, history):
+    """One rank's test users (int64 LOCAL rows) and held-out recipes (int64 GLOBAL ids) on its device, its history CSR
+    over local rows (None if it has none) and int64 [3] = (users, a user outside the rows that hold one, no history)
+    for the MAX all-reduce before any other collective.  Host and device users are checked there, without a wait."""
+    dev = g.device
+    u, h = (x.to(dev, torch.int64).reshape(-1) if torch.is_tensor(x) else
+            torch.as_tensor(np.asarray(x, np.int64).reshape(-1)).to(dev) for x in (users_local, held_out_global))
+    if h.numel() != u.numel():
+        raise ValueError(f"{h.numel()} held-out recipes for {u.numel()} test users")
+    if history is None:
+        hist = getattr(g.e, "_history", None)
+    else:
+        hist = tuple(torch.as_tensor(x).to(dev) for x in exclusion_csr(history, g.e.U))
+    flags = torch.tensor([u.numel(), 0, int(hist is None)], dtype=torch.int64, device=dev)
+    flags[1] = ((u < 0) | (u >= g.U_valid)).any()
+    return u, h, hist, flags
+
+
+def _full_ranking_check(flags):
+    """Raise what any rank found (``flags``: the reduced ``_full_ranking_inputs`` flags); else the most users a rank has."""
+    n_max, bad_user, no_history = (int(x) for x in flags.cpu())
+    if no_history:
+        raise L.FoodRecError("full ranking excludes each user's training recipes: pass history= or call "
+                             "ShardedEngine.set_user_history on every rank")
+    if bad_user:
+        raise IndexError("full ranking: a test user lies outside the rows of its shard that hold a user")
+    return n_max
+
+
+def _round_lists(u, h, hist, lo, hi, rn):
+    """The rn query rows of one round -- users lo:hi, then local row 0 as padding -- and their exclusion CSR: a user's
+    history row without its held-out recipe, an empty list for a padding row."""
+    off, ids = hist
+    dev = u.device
+    m = hi - lo
+    uu = torch.zeros(rn, dtype=torch.int32, device=dev)
+    uu[:m] = u[lo:hi]
+    held = torch.full((rn,), -1, dtype=torch.int64, device=dev)
+    held[:m] = h[lo:hi]
+    start = torch.zeros(rn, dtype=torch.int64, device=dev)
+    length = torch.zeros(rn, dtype=torch.int64, device=dev)
+    start[:m] = off[u[lo:hi]].long()
+    length[:m] = off[u[lo:hi] + 1].long() - start[:m]
+    total = int(length.sum())
+    row = torch.repeat_interleave(torch.arange(rn, device=dev), length, output_size=total)
+    first = torch.cumsum(length, 0) - length
+    vals = ids[start[row] + torch.arange(total, device=dev) - first[row]]
+    keep = vals.long() != held[row]
+    xoff = torch.zeros(rn + 1, dtype=torch.int32, device=dev)
+    xoff[1:] = torch.cumsum(torch.bincount(row[keep], minlength=rn), 0)
+    return uu, (xoff, vals[keep].to(torch.int32).contiguous())
+
+
+def _positions(ids, h):
+    """Position of h[j] in the merged list ids[j] ([m, K], -1 padded), -1 where it is absent."""
+    hit = (ids.long() == h[:, None]) & (h[:, None] >= 0)
+    return torch.where(hit.any(1), hit.int().argmax(1), -1).to(torch.int32)
 
 
 def concat_csr(lens, ids):
@@ -762,3 +848,19 @@ class LocalRunner:
                 g.eval_rank(u[lo:hi], rb, K, ids[lo:hi], rank[lo:hi], None if sc is None else sc[lo:hi])
         _eval_check_flag(torch.cat(flags))
         return [o if return_scores else o[:2] for o in outs]
+
+    def full_ranking(self, users_per_rank, held_per_rank, K, history=None, round_users=FULL_RANKING_ROUND_USERS):
+        """Same protocol as DistRunner.full_ranking with the collectives as tensor shuffles.  ``users_per_rank``,
+        ``held_per_rank`` and ``history`` (or None) hold one entry per rank.  Returns one int32 [n_r] per rank."""
+        hist = history if history is not None else [None] * self.W
+        ins = [_full_ranking_inputs(g, u, h, x) for g, u, h, x in zip(self.engs, users_per_rank, held_per_rank, hist)]
+        n_max = _full_ranking_check(torch.stack([f.cpu() for *_, f in ins]).max(0).values)
+        rn = max(1, min(int(round_users), n_max))
+        pos = [torch.full((u.numel(),), -1, dtype=torch.int32, device=u.device) for u, *_ in ins]
+        for a in range(0, n_max, rn):
+            span = [(min(a, u.numel()), min(a + rn, u.numel())) for u, *_ in ins]
+            lists = [_round_lists(u, h, x, lo, hi, rn) for (u, h, x, _), (lo, hi) in zip(ins, span)]
+            outs = self.catalog_topk([uu for uu, _ in lists], K, exclude=[ex for _, ex in lists])
+            for (_, h, _, _), (lo, hi), (ids, _), p in zip(ins, span, outs, pos):
+                p[lo:hi] = _positions(ids[:hi - lo], h[lo:hi])
+        return pos
